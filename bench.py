@@ -2,6 +2,7 @@
 """bench.py -- env-steps/sec of the adversarial-imitation round (BASELINE.json metric).
 
     python bench.py --gpus N --steps K --warmup W [--impl ours|reference] [--config hc|cartpole|airl_hc|ant|pref]
+                    [--dump-outputs DIR]
 
 A "step" is one ROUND of the reference's hot path (AdversarialTrainer.train body, algorithms/adversarial/common.py:453-461):
 generator rollout of E*T env steps with learned-reward relabel -> PPO update (n_epochs x minibatches) -> replay store ->
@@ -11,9 +12,14 @@ scripts/config/tuned_hps/gail_seals_half_cheetah_best_hp_eval.json, E = 1024 env
 scaling: every extra GPU adds 1024 envs.  The other BASELINE configs are selectable with --config (`pref` = reward-model
 training of preference comparisons, a different unit: fragment-pair evaluations / s).
 
-value   whole-job env-steps/s with everything resident in HBM (the captured-graph round); median of 5 timed windows of K rounds.
+value   whole-job env-steps/s with everything resident in HBM (the captured-graph round): K timed rounds, split into up to
+        --windows windows; the median of the windows' per-round times.
 e2e     the same metric through the reference-facing API with HOST expert batches: every train_disc() gets `expert_samples`
-        from pinned host memory (H2D inside the timed region) and returns its Mapping[str, float] (D2H inside the timed region).
+        from pinned host memory (H2D inside the timed region) and returns its Mapping[str, float] (D2H inside the timed region);
+        K timed rounds in up to 3 windows.
+--dump-outputs DIR  after the K timed captured-graph rounds, write what the last one left to its caller as DIR/<name>.npy
+        (float32 / float64): the round's discriminator statistics [n_disc, 16] and the trained policy and reward network
+        (state_dict entries).  Seeds are fixed, so two builds run with the same arguments can be compared output for output.
 roofline  dominant kernel by time share (the persistent PPO update); `roofline_disc`: the tcgen05 discriminator kernel on a
         2^20-row sweep point (tensor-pipe % from the committed ncu capture); `roofline_stages`: achieved GB/s of the stage-1/2
         kernels (rollout, sample+gather, ring store), all against MEASURED_PEAKS.json.
@@ -34,6 +40,7 @@ import torch as th
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: leave no __pycache__ in it
 
 # Per-GPU sizes (weak scaling).  `ppo`: SB3 PPO keyword arguments of the tuned JSON / script defaults.
 CONFIGS = {
@@ -413,20 +420,44 @@ def disc_roofline(tr, peak, device):
                     "(128 KB) fits in shared memory (profiles/r02_summary.md)"}
 
 
+def split_rounds(k: int, windows: int) -> list:
+    """k timed rounds over min(windows, k) windows of near-equal size."""
+    n = max(1, min(windows, k))
+    return [k // n + (i < k % n) for i in range(n)]
+
+
+def dump_outputs(tr, round_stats, out_dir):
+    """What one captured-graph round leaves to its caller: the round's discriminator statistics and the trained policy and
+    reward network, as float32 / float64 .npy files (integer buffers as float64)."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"round_stats": round_stats}
+    for prefix, module in (("policy", tr.policy), ("reward_net", tr.reward_train)):
+        arrays.update({f"{prefix}.{k}": v for k, v in module.state_dict().items()})
+    for name, v in arrays.items():
+        a = v.detach().cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a if a.dtype in (np.float32, np.float64) else a.astype(np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=200, help="timed rounds (each metric times this many)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="hc", choices=sorted(CONFIGS) + ["pref"])
     ap.add_argument("--cpu-rounds", type=int, default=12, help="rounds of the CPU baseline sample (rank 0, N=1)")
     ap.add_argument("--host-threads", type=int, default=4,
                     help="torch intra-op threads for the host side of the loop (all its CPU ops are tiny; the default pool of one thread per core makes the DataLoader-style shuffle ~30x slower); 0: leave torch default")
-    ap.add_argument("--windows", type=int, default=5, help="timed windows of --steps rounds each; the median is reported")
+    ap.add_argument("--windows", type=int, default=5,
+                    help="windows the --steps timed rounds are split into; the median per-round time is reported")
     ap.add_argument("--no-pin", action="store_true", help="do not pin the rank to its GPU's NUMA node")
     ap.add_argument("--profile-host", action="store_true", help="wall-clock breakdown of the e2e loop (every rank -> stderr)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed round's outputs to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.config == "pref" or args.impl != "ours"):
+        ap.error("--dump-outputs writes the outputs of the GPU adversarial round (--impl ours, not --config pref)")
     if args.config == "pref":
         import importlib.util
 
@@ -522,17 +553,17 @@ def main():
         round_graph()
     th.cuda.synchronize()
 
-    # ---- value: windows of K graph-replayed rounds, device timed, max over ranks, median over windows ----------------
+    # ---- value: K graph-replayed rounds in windows, device timed, max over ranks, median per-round time over windows ----
     K = args.steps
-    win_ms = []
+    win_ms, win_rounds, launches = [], split_rounds(K, args.windows), 0
     with ClockSampler(local, enabled=(rank == 0)) as clocks:
-        for _ in range(max(1, args.windows)):
+        for k in win_rounds:
             if world > 1:
                 dist.barrier()
             th.cuda.synchronize()
             l0 = _lib.LAUNCHES["count"]
-            ms = cuda_time_ms(lambda: [round_graph() for _ in range(K)])
-            launches = _lib.LAUNCHES["count"] - l0
+            ms = cuda_time_ms(lambda: [round_graph() for _ in range(k)])
+            launches += _lib.LAUNCHES["count"] - l0
             th.cuda.synchronize()
             if world > 1:
                 t = th.tensor([ms], device=device)
@@ -541,8 +572,10 @@ def main():
             win_ms.append(ms)
         if world > 1:
             dist.barrier()
-    ms = statistics.median(win_ms)
-    value = world * E * T * K / (ms / 1e3)
+    ms_round = statistics.median(m / k for m, k in zip(win_ms, win_rounds))
+    value = world * E * T / (ms_round / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(tr, tr._round_stats, args.dump_outputs)
 
     # ---- e2e: reference-facing API, host expert batches, stats read back every update ---------------------------
     # Host side = what a DataLoader(shuffle=True, drop_last=True) does: the demonstrations live in pinned
@@ -600,7 +633,6 @@ def main():
             tr.join()
             sync.end_round()
 
-    Ke = max(3, min(K, 50))
     for _ in range(3):
         round_e2e()
     th.cuda.synchronize()
@@ -640,19 +672,19 @@ def main():
         for k, v in sorted(acc.items(), key=lambda kv: -kv[1]):
             msg += f"[rank {rank}]   {k:<20s} {v * 100:.3f} ms/round\n"
         sys.stderr.write(msg)
-    e2e_ms = []
-    for _ in range(3):
+    e2e_ms, e2e_rounds = [], split_rounds(K, 3)
+    for k in e2e_rounds:
         if world > 1:
             dist.barrier()
         th.cuda.synchronize()
-        ms_e = cuda_time_ms(lambda: [round_e2e() for _ in range(Ke)])
+        ms_e = cuda_time_ms(lambda: [round_e2e() for _ in range(k)])
         if world > 1:
             t = th.tensor([ms_e], device=device)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms_e = float(t)
         e2e_ms.append(ms_e)
-    ms_e = statistics.median(e2e_ms)
-    e2e_value = world * E * T * Ke / (ms_e / 1e3)
+    ms_e = statistics.median(m / k for m, k in zip(e2e_ms, e2e_rounds))
+    e2e_value = world * E * T / (ms_e / 1e3)
 
     # ---- roofline: dominant kernel (PPO update) + disc kernel sweep point + stage kernels (rank 0) ------------------------------
     roof, roof_disc, roof_stages, cpu_base = None, None, None, None
@@ -676,7 +708,7 @@ def main():
                 # configuration (profiles/ncu_ppo_r02c_selected.csv, the kernel as it is at the end of round 2): the rollout
                 # table stays in L2
                 "traffic": PPO_DRAM_BYTES_NCU if args.config == "hc" else None,
-                "peak_source": peak_src, "ms_per_launch": ms_ppo, "share_of_step": ms_ppo / (ms / K),
+                "peak_source": peak_src, "ms_per_launch": ms_ppo, "share_of_step": ms_ppo / ms_round,
                 "algorithmic_bytes_per_launch": ppo_bytes,
                 "note": f"latency-bound by construction: {n_opt} dependent optimiser steps of {cfg['ppo_minibatch']} rows each; "
                         "the HBM fraction is reported as required, the figure of merit is us per minibatch step = "
@@ -693,12 +725,13 @@ def main():
     if rank == 0:
         line = {"metric": "GAIL env-steps/sec (disc+gen loop)" if cfg["algo"] == "gail" else "AIRL env-steps/sec (disc+gen loop)",
                 "value": value, "unit": "env-steps/s",
-                "n_gpus": world, "steps": K, "warmup": W, "ms_per_step": ms / K,
-                "windows_ms": [round(x, 4) for x in win_ms],
+                "n_gpus": world, "steps": K, "warmup": W, "ms_per_step": ms_round,
+                "windows_ms": [round(x, 4) for x in win_ms], "windows_steps": win_rounds,
                 "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
                 "config": config, "clocks": clocks.summary(),
                 "e2e": {"value": e2e_value, "unit": "env-steps/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h,
-                        "steps": Ke, "ms_per_step": ms_e / Ke, "windows_ms": [round(x, 4) for x in e2e_ms],
+                        "steps": K, "ms_per_step": ms_e, "windows_ms": [round(x, 4) for x in e2e_ms],
+                        "windows_steps": e2e_rounds,
                         "path": f"{cfg['algo'].upper()}.train_gen() + .train_disc(expert_samples=<pinned host batch>) -> "
                                 "Mapping[str,float]"},
                 "gpu_launches": launches, "roofline": roof, "roofline_disc": roof_disc, "roofline_stages": roof_stages,

@@ -5,7 +5,8 @@ TEST INFRASTRUCTURE.  Runs only in the build container (needs /root/reference):
 The reference is imported unchanged from /root/reference/src through the names-only
 shim (oracle/_shim); every stored output is produced by reference code:
   algorithms/adversarial/{common,gail,airl}.py, rewards/reward_nets.py, util/networks.py,
-  data/{buffer,wrappers,rollout}.py, rewards/reward_wrapper.py, algorithms/base.py.
+  data/{buffer,wrappers,rollout,serialize,types}.py, rewards/{reward_wrapper,serialize}.py, algorithms/base.py,
+  algorithms/preference_comparisons.py, util/util.py.
 The fixtures pin (a) the CPU restatement in oracle/*_port.py and (b) the CUDA path.
 """
 import os
@@ -17,6 +18,9 @@ import torch as th
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(HERE))
 from oracle import refimport, synth_env  # noqa: E402
+from oracle.api_cases import (HORIZON_SCRIPTS, PREF_SETTINGS, ROLLOUT_LENS, SAMPLE_UNTIL, SAMPLE_UNTIL_BAD,  # noqa: E402
+                              SCHEDULE_RUNS, error, make_dataset_trajectories, make_hf_trajectories,
+                              make_rollout_trajectories, validation_cases)
 
 refimport.load()
 from gymnasium import spaces  # noqa: E402  (shim)
@@ -338,6 +342,139 @@ def preference_case():
     print("wrote preference")
 
 
+def reference_api_case():
+    """Host-side API of the reference on seeded inputs, for tests/test_oracle_vs_reference.py: data/serialize.py's
+    demonstration directories, data/rollout.py helpers, algorithms/base.py's fixed-horizon check, data/types.py
+    validation messages, preference_comparisons.py schedules / datasets / PreferenceModel, util/util.py oric and
+    make_seeds, reward_nets.py preprocess and the reward registry, util/networks.py RunningNorm.
+    Arrays go to reference_api.npz; everything else as one JSON document under its `facts` key."""
+    import json
+    import shutil
+
+    from imitation.algorithms import preference_comparisons as ref_pc
+    from imitation.data import serialize as ref_serialize
+    from imitation.rewards import serialize as ref_ser
+
+    out, facts = {}, {}
+    # demonstration directories written by the reference (data/serialize.py:15-24)
+    rng = np.random.default_rng(3)
+    for discrete in (False, True):
+        path = os.path.join(OUT, f"hf_reference_{int(discrete)}")
+        shutil.rmtree(path, ignore_errors=True)
+        ref_serialize.save(path, make_hf_trajectories(ref_types, rng, discrete))
+    # rollout helpers (data/rollout.py:193-286, 509-621, 728-745)
+    rng = np.random.default_rng(5)
+    for monitor in (False, True):
+        trajs = make_rollout_trajectories(ref_types, rng, monitor)
+        facts[f"rollout_stats/{int(monitor)}"] = ref_rollout.rollout_stats(trajs)
+        flat = ref_rollout.flatten_trajectories_with_rew(trajs)
+        for field in ("obs", "acts", "next_obs", "dones", "rews"):
+            out[f"flatten/{int(monitor)}/{field}"] = getattr(flat, field)
+        facts[f"sample_until/{int(monitor)}"] = [bool(ref_rollout.make_sample_until(**kw)(trajs)) for kw in SAMPLE_UNTIL]
+    facts["sample_until_errors"] = [error(lambda: ref_rollout.make_sample_until(**kw)) for kw in SAMPLE_UNTIL_BAD]
+    arr = rng.standard_normal((7, 3))
+    out["discounted_sum/input"] = arr
+    for gamma in (1.0, 0.9):
+        out[f"discounted_sum/{gamma}/2d"] = ref_rollout.discounted_sum(arr, gamma)
+        out[f"discounted_sum/{gamma}/1d"] = ref_rollout.discounted_sum(arr[:, 0], gamma)
+    # fixed-horizon check (algorithms/base.py:69-108): per step ["ok", remembered horizon] or ["err", message]
+    for allow in (False, True):
+        runs = []
+        for script in HORIZON_SCRIPTS:
+            algo, events = ref_base.BaseImitationAlgorithm(allow_variable_horizon=allow), []
+            for horizons in script:
+                try:
+                    algo._check_fixed_horizon(horizons)
+                except ValueError as e:
+                    events.append(["err", str(e)])
+                    break
+                events.append(["ok", algo._horizon])
+            runs.append(events)
+        facts[f"fixed_horizon/{int(allow)}"] = runs
+    # validation messages (data/types.py:61-330)
+    cases, ok = validation_cases()
+    facts["validation"] = {name: error(lambda: getattr(ref_types, cls)(**kw)) for name, (cls, kw) in cases.items()}
+    facts["transitions_len"] = len(ref_types.Transitions(**ok))
+    # comparison schedule (util.oric, make_seeds, QUERY_SCHEDULES; preference_comparisons.py:1465-1479, 1622-1636)
+    rng = np.random.default_rng(0)
+    oric = []
+    for _ in range(500):
+        n, total = int(rng.integers(1, 12)), int(rng.integers(0, 300))
+        v = rng.random(n) + 1e-3
+        oric.append(ref_util.oric(v / v.sum() * total).tolist())
+    facts["oric"] = oric
+    facts["make_seeds"] = [ref_util.make_seeds(np.random.default_rng(9), n) for n in (None, 1, 5)]
+    facts["query_schedules"] = {name: [fn(t) for t in np.linspace(0, 1, 7)] for name, fn in ref_pc.QUERY_SCHEDULES.items()}
+    facts["schedule_runs"] = {}
+    for name, fn in ref_pc.QUERY_SCHEDULES.items():
+        for total, iters, frac in SCHEDULE_RUNS:
+            initial = int(total * frac)
+            vec = np.array([fn(t) for t in np.linspace(0, 1, iters)])
+            facts["schedule_runs"][f"{name}/{total}/{iters}/{frac}"] = \
+                [initial] + ref_util.oric(vec / vec.sum() * (total - initial)).tolist()
+    # RewardNet.preprocess and the reward-loader registry (reward_nets.py:74-118, rewards/serialize.py:230-260)
+    facts["reward_registry"] = sorted(ref_ser.reward_registry.keys())
+    rng = np.random.default_rng(0)
+    for discrete in (True, False):
+        net = ref_nets.BasicRewardNet(spaces.Box(-1, 1, (4,)), spaces.Discrete(3) if discrete else spaces.Box(-1, 1, (2,)))
+        obs, nobs = rng.standard_normal((6, 4)), rng.standard_normal((6, 4)).astype(np.float32)
+        acts = rng.integers(0, 3, 6) if discrete else rng.uniform(-1, 1, (6, 2))
+        done = rng.random(6) < 0.5
+        pre = net.preprocess(obs, acts, nobs, done)
+        facts[f"preprocess/{int(discrete)}/dtypes"] = [str(t.dtype) for t in pre]
+        for i, t in enumerate(pre):
+            out[f"preprocess/{int(discrete)}/{i}"] = t.numpy()
+        facts[f"state_dict_shapes/{int(discrete)}"] = {k: list(v.shape) for k, v in net.state_dict().items()}
+    # TrajectoryDataset.sample / PreferenceDataset (preference_comparisons.py:99-124, 909-997)
+    trajs = make_dataset_trajectories(ref_types)
+    tds = ref_pc.TrajectoryDataset(trajs, np.random.default_rng(7))
+    for steps in (10, 25, 46, 1):
+        sample = tds.sample(steps)
+        facts[f"trajectory_sample/{steps}/lens"] = [len(t) for t in sample]
+        out[f"trajectory_sample/{steps}/obs"] = np.concatenate([t.obs for t in sample])
+    facts["trajectory_sample_error"] = error(lambda: tds.sample(100), RuntimeError)
+    pds = ref_pc.PreferenceDataset(max_size=3)
+    f = trajs
+    pds.push([(f[0], f[1]), (f[2], f[3])], np.array([1.0, 0.0], np.float32))
+    pds.push([(f[4], f[5]), (f[6], f[0])], np.array([0.5, 1.0], np.float32))
+    facts["preference_dataset_len"] = len(pds)
+    out["preference_dataset/preferences"] = pds.preferences
+    for i in range(3):
+        (x, y), p = pds[i]
+        out[f"preference_dataset/{i}/pref"], out[f"preference_dataset/{i}/x_obs"] = np.asarray(p), x.obs
+        out[f"preference_dataset/{i}/y_acts"] = y.acts
+    facts["preference_dataset_errors"] = [error(lambda: pds.push([(f[0], f[1]), (f[2], f[3])], bad))
+                                          for bad in (np.array([1.0], np.float32), np.array([1.0, 0.0], np.float64))]
+    # RunningNorm over training batches, then in eval mode (util/networks.py:19-134)
+    norm = ref_networks.RunningNorm(5)
+    g = th.Generator().manual_seed(0)
+    for step in range(5):
+        y = norm(th.randn(7 + step, 5, generator=g) * (1 + step) + step)
+        out[f"running_norm/{step}/y"] = y.numpy()
+        out.update(_flat(f"running_norm/{step}/state", _state(norm)))
+    norm.eval()
+    out["running_norm/eval/y"] = norm(th.randn(3, 5, generator=g)).numpy()
+    out.update(_flat("running_norm/eval/state", _state(norm)))
+    facts["running_norm_dtypes"] = {k: str(v.dtype) for k, v in norm.state_dict().items()}
+    # PreferenceModel.probability and the cross-entropy loss (preference_comparisons.py:487-530, 1043-1090)
+    net = ref_nets.BasicRewardNet(spaces.Box(-1, 1, (4,)), spaces.Box(-1, 1, (2,)))
+    g = th.Generator().manual_seed(0)
+    for i, (noise, discount, threshold) in enumerate(PREF_SETTINGS):
+        pm = ref_pc.PreferenceModel(net, noise_prob=noise, discount_factor=discount, threshold=threshold)
+        for scale in (0.3, 3.0):
+            r1, r2 = th.randn(12, generator=g) * scale, th.randn(12, generator=g) * scale
+            out[f"probability/{i}/{scale}"] = pm.probability(r1, r2).numpy()
+        R1, R2 = th.randn(9, 12, generator=g) * 2, th.randn(9, 12, generator=g) * 2
+        single = th.stack([pm.probability(x, y) for x, y in zip(R1, R2)])
+        prefs = (th.rand(9, generator=g) < 0.5).float()
+        out[f"probability/{i}/pairs"] = single.numpy()
+        out[f"probability/{i}/bce"] = th.nn.functional.binary_cross_entropy(single, prefs).numpy()
+        out[f"probability/{i}/accuracy"] = ((single > 0.5) == (prefs > 0.5)).float().mean().numpy()
+    out["facts"] = np.array(json.dumps(facts, sort_keys=True))
+    np.savez_compressed(os.path.join(OUT, "reference_api.npz"), **out)
+    print("wrote reference_api")
+
+
 def all_cases():
     """Every golden file of tests/golden/, (name, thunk) in generation order (shared with
     tests/test_oracle_vs_reference.py, which regenerates ALL of them from the reference)."""
@@ -362,6 +499,7 @@ def all_cases():
         ("expert_loader", expert_loader_case),
         ("train_stats", train_stats_case),
         ("preference", preference_case),
+        ("reference_api", reference_api_case),
     ]
 
 

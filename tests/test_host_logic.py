@@ -204,16 +204,14 @@ def test_demo_ingest_reads_legacy_npz_fixture(name):
     assert len(trajs) in (3, 4)
 
 
-@pytest.mark.refsrc
 @pytest.mark.parametrize("rel", ["cartpole_0/rollouts/final.npz", "pendulum_0/rollouts/final.npz"])
 def test_demo_ingest_reads_reference_rollouts(rel):
-    """The reference's full on-disk demonstrations (27 k CartPole / 11 k Pendulum transitions; container only)."""
+    """Every trajectory of the reference's on-disk expert demonstrations (57 CartPole / 56 Pendulum episodes), each cut
+    to its first 8 transitions (oracle/make_demo_fixture.py)."""
     import os
 
-    path = os.path.join("/root/reference/tests/testdata/expert_models", rel)
-    if not os.path.exists(path):
-        pytest.skip("reference checkout not present")
-    trajs = _check_fixture(path)
+    name = {"cartpole_0/rollouts/final.npz": "demo_cartpole_all", "pendulum_0/rollouts/final.npz": "demo_pendulum_all"}[rel]
+    trajs = _check_fixture(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", name + ".npz"))
     assert len(trajs) > 50
 
 

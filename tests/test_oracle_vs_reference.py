@@ -1,20 +1,259 @@
-"""Build-container only: regenerate the golden vectors from the REAL reference
-(/root/reference/src, imported through oracle/_shim) and check they equal the committed
-fixtures -- i.e. tests/golden/*.npz really are outputs of the reference's own modules.
-Skipped where /root/reference does not exist (the GPU box)."""
+"""This repository's host-side API against the reference's: the reference's own functions were run on the seeded inputs of
+oracle/api_cases.py by oracle/make_golden.py, and what they returned is stored in tests/golden/reference_api.npz (the
+demonstration directories it wrote in tests/golden/hf_reference_*).  Each test runs this repository's functions on the
+same inputs and compares.
+
+The last three tests check the provenance of the fixtures themselves -- they regenerate them from the reference's sources
+(imported through oracle/_shim) -- and skip where those sources are not present."""
+import json
 import os
 
 import numpy as np
 import pytest
 
 from oracle import refimport
-
-pytestmark = [pytest.mark.refsrc,
-              pytest.mark.skipif(not refimport.available(), reason="/root/reference not present")]
+from oracle.api_cases import (HORIZON_SCRIPTS, PREF_SETTINGS, SAMPLE_UNTIL, SAMPLE_UNTIL_BAD, SCHEDULE_RUNS, error,
+                              make_dataset_trajectories, make_hf_trajectories, make_rollout_trajectories, validation_cases)
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+REF = np.load(os.path.join(GOLDEN, "reference_api.npz"))
+FACTS = json.loads(str(REF["facts"]))
 
 
+def test_huggingface_demonstration_format_is_interchangeable_with_the_reference(tmp_path):
+    """f3: a demonstration directory written by the REFERENCE's `data.serialize.save` (its `huggingface_utils` over the real
+    `datasets` package) is read by `imitation_b200.data.serialize.load`, and this repo's `save` writes the same dataset
+    (features and rows) as the reference for the same trajectories -- so the reference's `load` reads it."""
+    datasets = pytest.importorskip("datasets")
+
+    from imitation_b200.data import serialize, types
+
+    def same(a, b):
+        assert len(a) == len(b)
+        for x, y in zip(a, b):
+            np.testing.assert_array_equal(np.asarray(x.obs, dtype=np.float32), np.asarray(y.obs, dtype=np.float32))
+            np.testing.assert_array_equal(np.asarray(x.acts), np.asarray(y.acts))
+            np.testing.assert_array_equal(np.asarray(x.rews, dtype=np.float32), np.asarray(y.rews, dtype=np.float32))
+            assert bool(x.terminal) == bool(y.terminal)
+            xi = [{}] * len(x.acts) if x.infos is None else list(x.infos)
+            yi = [{}] * len(y.acts) if y.infos is None else list(y.infos)
+            assert xi == yi
+
+    rng = np.random.default_rng(3)
+    for discrete in (False, True):
+        trajs = make_hf_trajectories(types, rng, discrete)
+        theirs = os.path.join(GOLDEN, f"hf_reference_{int(discrete)}")
+        same(trajs, serialize.load_with_rewards(theirs))                   # the reference wrote, this repo reads
+        serialize.save(tmp_path / f"ours_{int(discrete)}", trajs)          # this repo writes what the reference wrote
+        ours, want = datasets.load_from_disk(str(tmp_path / f"ours_{int(discrete)}")), datasets.load_from_disk(theirs)
+        assert ours.features == want.features
+        assert ours.to_dict() == want.to_dict()
+        same(trajs, serialize.load_with_rewards(tmp_path / f"ours_{int(discrete)}"))
+
+
+def test_host_side_rollout_helpers_agree_with_the_reference():
+    """f4: `rollout_stats` (with and without Monitor infos), `discounted_sum`, the sample-until predicates and
+    `flatten_trajectories_with_rew` of imitation_b200.data.rollout against the reference's own functions
+    (data/rollout.py:193-286, 509-621, 728-745) on the same random trajectories."""
+    from imitation_b200.data import rollout, types
+
+    rng = np.random.default_rng(5)
+    for monitor in (False, True):
+        ours = make_rollout_trajectories(types, rng, monitor)
+        want, got = FACTS[f"rollout_stats/{int(monitor)}"], rollout.rollout_stats(ours)
+        assert set(got) == set(want) and ("monitor_return_mean" in want) == monitor
+        for k in want:
+            assert got[k] == want[k] and type(got[k]) is type(want[k]), k
+        fg = rollout.flatten_trajectories_with_rew(ours)
+        for field in ("obs", "acts", "next_obs", "dones", "rews"):
+            np.testing.assert_array_equal(getattr(fg, field), REF[f"flatten/{int(monitor)}/{field}"], err_msg=field)
+        assert [rollout.make_sample_until(**kw)(ours) for kw in SAMPLE_UNTIL] == FACTS[f"sample_until/{int(monitor)}"]
+    assert [error(lambda: rollout.make_sample_until(**kw)) for kw in SAMPLE_UNTIL_BAD] == FACTS["sample_until_errors"]
+    arr = rng.standard_normal((7, 3))
+    np.testing.assert_array_equal(arr, REF["discounted_sum/input"])
+    for gamma in (1.0, 0.9):
+        np.testing.assert_allclose(rollout.discounted_sum(arr, gamma), REF[f"discounted_sum/{gamma}/2d"], rtol=1e-12)
+        np.testing.assert_allclose(rollout.discounted_sum(arr[:, 0], gamma), REF[f"discounted_sum/{gamma}/1d"], rtol=1e-12)
+
+
+def test_fixed_horizon_check_agrees_with_the_reference():
+    """a21: BaseImitationAlgorithm._check_fixed_horizon (algorithms/base.py:69-108): same accept / reject decisions, same
+    remembered horizon and the same error text as the reference's class over sequences of episode lengths."""
+    from imitation_b200.algorithms import base
+
+    class Ours(base.BaseImitationAlgorithm):
+        pass
+
+    for allow in (False, True):
+        for script, want in zip(HORIZON_SCRIPTS, FACTS[f"fixed_horizon/{int(allow)}"]):
+            algo, events = Ours(allow_variable_horizon=allow), []
+            for horizons in script:
+                try:
+                    algo._check_fixed_horizon(horizons)
+                except ValueError as e:
+                    events.append(["err", str(e)])
+                    break
+                events.append(["ok", algo._horizon])
+            assert events == want, (allow, script)
+
+
+def test_trajectory_and_transition_validation_agrees_with_the_reference():
+    """data/types.py:61-330: the same inputs are rejected with the same messages by this repo's Trajectory / TrajectoryWithRew /
+    Transitions and by the reference's."""
+    from imitation_b200.data import types as M
+
+    cases, ok = validation_cases()
+    for name, (cls, kw) in cases.items():
+        assert error(lambda: getattr(M, cls)(**kw)) == FACTS["validation"][name], name
+    assert len(M.Transitions(**ok)) == FACTS["transitions_len"] == 3
+
+
+def test_comparison_schedule_helpers_agree_with_the_reference():
+    """f1: the per-iteration comparison counts of PreferenceComparisons.train (preference_comparisons.py:1622-1636) --
+    `util.oric` rounding of the query-schedule shares -- and the named query schedules (:1465-1479)."""
+    from imitation_b200.algorithms import preference_comparisons as pc
+
+    rng = np.random.default_rng(0)
+    for want in FACTS["oric"]:
+        n, total = int(rng.integers(1, 12)), int(rng.integers(0, 300))
+        v = rng.random(n) + 1e-3
+        x = v / v.sum() * total
+        np.testing.assert_array_equal(pc._round_keep_sum(x), np.array(want, dtype=np.int64))
+    # seeds handed to samplers / DataLoaders come from the caller's generator the same way
+    assert [pc.make_seeds(np.random.default_rng(9), n) for n in (None, 1, 5)] == FACTS["make_seeds"]
+    assert set(pc.QUERY_SCHEDULES) == set(FACTS["query_schedules"])
+    for name, fn in pc.QUERY_SCHEDULES.items():
+        assert [fn(t) for t in np.linspace(0, 1, 7)] == FACTS["query_schedules"][name], name
+    # the whole schedule of a run: initial comparisons + oric(shares), as PreferenceComparisons.train computes it
+    for name in pc.QUERY_SCHEDULES:
+        for total, iters, frac in SCHEDULE_RUNS:
+            initial = int(total * frac)
+            vec = np.array([pc.QUERY_SCHEDULES[name](t) for t in np.linspace(0, 1, iters)])
+            ours = [initial] + [int(v) for v in pc._round_keep_sum(vec / vec.sum() * (total - initial))]
+            assert ours == FACTS["schedule_runs"][f"{name}/{total}/{iters}/{frac}"] and sum(ours) == total
+
+
+def test_reward_net_preprocess_and_registry_agree_with_the_reference():
+    """a8 / f4: `RewardNet.preprocess` (reward_nets.py:74-118: float conversion, one-hot Discrete actions) on CPU tensors and
+    the registered reward-loader names of rewards/serialize.py:230-260 against the reference's."""
+    import torch as th
+
+    from imitation_b200 import spaces
+    from imitation_b200.rewards import reward_nets, serialize
+
+    assert sorted(serialize.reward_registry.keys()) == FACTS["reward_registry"]
+    rng = np.random.default_rng(0)
+    for discrete in (True, False):
+        ours = reward_nets.BasicRewardNet(spaces.Box(-1, 1, (4,)), spaces.Discrete(3) if discrete else spaces.Box(-1, 1, (2,)))
+        obs, nobs = rng.standard_normal((6, 4)), rng.standard_normal((6, 4)).astype(np.float32)
+        acts = rng.integers(0, 3, 6) if discrete else rng.uniform(-1, 1, (6, 2))
+        done = rng.random(6) < 0.5
+        got = ours.preprocess(obs, acts, nobs, done)
+        assert [str(a.dtype) for a in got] == FACTS[f"preprocess/{int(discrete)}/dtypes"]
+        for i, a in enumerate(got):
+            assert th.equal(a, th.as_tensor(REF[f"preprocess/{int(discrete)}/{i}"]))
+        assert {k: list(v.shape) for k, v in ours.state_dict().items()} == FACTS[f"state_dict_shapes/{int(discrete)}"]
+
+
+def test_trajectory_dataset_and_preference_dataset_agree_with_the_reference(tmp_path):
+    """f1 host side: `TrajectoryDataset.sample` (preference_comparisons.py:99-124: shuffled selection with the caller's
+    generator), `PreferenceDataset` FIFO / pickling (:909-997) against the reference's classes for the same seeds."""
+    from imitation_b200.algorithms import preference_comparisons as pc
+    from imitation_b200.data import types
+
+    ours = make_dataset_trajectories(types)
+    b = pc.TrajectoryDataset(ours, np.random.default_rng(7))
+    for steps in (10, 25, 46, 1):
+        tb = b.sample(steps)
+        assert [len(t) for t in tb] == FACTS[f"trajectory_sample/{steps}/lens"]
+        np.testing.assert_array_equal(np.concatenate([t.obs for t in tb]), REF[f"trajectory_sample/{steps}/obs"])
+    assert error(lambda: b.sample(100), RuntimeError) == FACTS["trajectory_sample_error"]
+    db, f = pc.PreferenceDataset(max_size=3), ours
+    db.push([(f[0], f[1]), (f[2], f[3])], np.array([1.0, 0.0], np.float32))
+    db.push([(f[4], f[5]), (f[6], f[0])], np.array([0.5, 1.0], np.float32))
+    assert len(db) == FACTS["preference_dataset_len"] == 3
+    np.testing.assert_array_equal(db.preferences, REF["preference_dataset/preferences"])
+    for i in range(3):
+        (xb, yb), pb = db[i]
+        assert pb == REF[f"preference_dataset/{i}/pref"]
+        assert np.array_equal(xb.obs, REF[f"preference_dataset/{i}/x_obs"])
+        assert np.array_equal(yb.acts, REF[f"preference_dataset/{i}/y_acts"])
+    db.save(tmp_path / "prefs.pkl")
+    back = pc.PreferenceDataset.load(tmp_path / "prefs.pkl")
+    assert len(back) == 3 and np.array_equal(back.preferences, db.preferences) and back.max_size == 3
+    msgs = [error(lambda: db.push([(f[0], f[1]), (f[2], f[3])], bad))
+            for bad in (np.array([1.0], np.float32), np.array([1.0, 0.0], np.float64))]
+    assert msgs == FACTS["preference_dataset_errors"]
+
+
+def test_running_norm_module_and_mode_helpers_agree_with_the_reference():
+    """a10: the torch-level `RunningNorm` module (util/networks.py:19-134; the API path and the policy's
+    NormalizeFeaturesExtractor use it on whatever device the tensors are on) is bit-identical to the reference's over a
+    sequence of training batches and in eval mode; `training()` / `evaluating()` context managers restore the mode."""
+    import torch as th
+
+    from imitation_b200.util import networks
+
+    def state_is(m, prefix):
+        for k, v in m.state_dict().items():
+            assert th.equal(v, th.as_tensor(REF[f"{prefix}/{k}"])), (prefix, k)
+
+    b = networks.RunningNorm(5)
+    g = th.Generator().manual_seed(0)
+    for step in range(5):
+        x = th.randn(7 + step, 5, generator=g) * (1 + step) + step
+        assert th.equal(b(x), th.as_tensor(REF[f"running_norm/{step}/y"]))
+        state_is(b, f"running_norm/{step}/state")
+    b.eval()
+    x = th.randn(3, 5, generator=g)
+    assert th.equal(b(x), th.as_tensor(REF["running_norm/eval/y"])) and int(b.count) == 45
+    state_is(b, "running_norm/eval/state")
+    assert {k: str(v.dtype) for k, v in b.state_dict().items()} == FACTS["running_norm_dtypes"]
+    prefix = "running_norm/eval/state/"
+    b.load_state_dict({k[len(prefix):]: th.as_tensor(REF[k]) for k in REF.files if k.startswith(prefix)})
+    for ctx, want in ((networks.training, True), (networks.evaluating, False)):
+        b.eval()
+        with ctx(b):
+            assert b.training is want
+        assert b.training is False
+        b.train()
+        with ctx(b):
+            assert b.training is want
+        assert b.training is True
+
+
+def test_preference_probability_and_loss_agree_with_the_reference():
+    """f1: `PreferenceModel.probability` (preference_comparisons.py:487-530: discounting, clipping at the threshold, noise
+    floor) and the cross-entropy / accuracy arithmetic of `CrossEntropyRewardLoss` (:1043-1090) on CPU tensors against the
+    reference's classes, for several (noise_prob, discount_factor, threshold) settings incl. clipped return differences."""
+    import torch as th
+
+    from imitation_b200 import spaces
+    from imitation_b200.algorithms import preference_comparisons as pc
+    from imitation_b200.rewards import reward_nets
+
+    ours_net = reward_nets.BasicRewardNet(spaces.Box(-1, 1, (4,)), spaces.Box(-1, 1, (2,)))
+    g = th.Generator().manual_seed(0)
+    for i, (noise, discount, threshold) in enumerate(PREF_SETTINGS):
+        b = pc.PreferenceModel(ours_net, noise_prob=noise, discount_factor=discount, threshold=threshold)
+        for scale in (0.3, 3.0):
+            r1, r2 = th.randn(12, generator=g) * scale, th.randn(12, generator=g) * scale
+            pb = b.probability(r1, r2)
+            assert pb.shape == () and th.equal(pb, th.as_tensor(REF[f"probability/{i}/{scale}"]))
+        # a batch of pairs the way the fused path lays it out: [P, L] rewards, time on axis 1
+        R1, R2 = th.randn(9, 12, generator=g) * 2, th.randn(9, 12, generator=g) * 2
+        batch = b._probability(R1, R2, time_axis=1)
+        single = th.as_tensor(REF[f"probability/{i}/pairs"])
+        th.testing.assert_close(batch, single, rtol=1e-6, atol=1e-7)
+        prefs = (th.rand(9, generator=g) < 0.5).float()
+        want = th.as_tensor(REF[f"probability/{i}/bce"])
+        th.testing.assert_close(th.nn.functional.binary_cross_entropy(batch, prefs), want, rtol=1e-6, atol=1e-7)
+        assert ((batch > 0.5) == (prefs > 0.5)).float().mean() == th.as_tensor(REF[f"probability/{i}/accuracy"])
+
+
+# ---- provenance of the fixtures: regenerated from the reference's sources ---------------------------------------------
+@pytest.mark.refsrc
+@pytest.mark.skipif(not refimport.available(), reason="reference sources not present")
 def test_goldens_reproduce_from_reference(tmp_path):
     """EVERY file under tests/golden/ is regenerated from the reference's own modules and compared with the committed
     fixture (no golden is taken on trust)."""
@@ -36,16 +275,24 @@ def test_goldens_reproduce_from_reference(tmp_path):
                 assert [str(x) for x in np.ravel(new[k])] == [str(x) for x in np.ravel(old[k])], f"{name}:{k}"
             else:
                 np.testing.assert_array_equal(new[k], old[k], err_msg=f"{name}:{k}")
+    datasets = pytest.importorskip("datasets")
+    for d in (0, 1):
+        new = datasets.load_from_disk(os.path.join(str(tmp_path), f"hf_reference_{d}"))
+        old = datasets.load_from_disk(os.path.join(GOLDEN, f"hf_reference_{d}"))
+        assert new.features == old.features and new.to_dict() == old.to_dict()
 
 
+@pytest.mark.refsrc
+@pytest.mark.skipif(not refimport.available(), reason="reference sources not present")
 def test_demo_fixtures_are_cut_from_the_reference_rollouts(tmp_path):
-    """tests/golden/demo_*.npz = leading trajectories of the reference's own expert rollouts (oracle/make_demo_fixture.py)."""
+    """tests/golden/demo_*.npz = leading trajectories, or every trajectory shortened, of the reference's own expert
+    rollouts (oracle/make_demo_fixture.py)."""
     from oracle import make_demo_fixture as mdf
 
-    for src, name, k in (("cartpole_0/rollouts/final.npz", "demo_cartpole_legacy", 4),
-                         ("pendulum_0/rollouts/final.npz", "demo_pendulum_legacy", 3)):
+    made = [(mdf.cut, src, k, name) for src, k, name in mdf.CUTS] + [(mdf.shrink, src, n, name) for src, n, name in mdf.SHRINKS]
+    for fn, src, k, name in made:
         out = os.path.join(str(tmp_path), name + ".npz")
-        mdf.cut(os.path.join(mdf.REF, src), out, k)
+        fn(os.path.join(mdf.REF, src), out, k)
         new, old = np.load(out, allow_pickle=True), np.load(os.path.join(GOLDEN, name + ".npz"), allow_pickle=True)
         assert set(new.files) == set(old.files)
         for key in old.files:
@@ -55,343 +302,11 @@ def test_demo_fixtures_are_cut_from_the_reference_rollouts(tmp_path):
                 np.testing.assert_array_equal(new[key], old[key], err_msg=f"{name}:{key}")
 
 
+@pytest.mark.refsrc
+@pytest.mark.skipif(not refimport.available(), reason="reference sources not present")
 def test_reference_modules_used_are_the_real_ones():
     im = refimport.load()
-    assert im.__file__.startswith("/root/reference/src/imitation")
+    assert im.__file__.startswith(os.path.join(refimport.REF_SRC, "imitation"))
     from imitation.algorithms.adversarial import common
 
-    assert common.__file__ == "/root/reference/src/imitation/algorithms/adversarial/common.py"
-
-
-def test_huggingface_demonstration_format_is_interchangeable_with_the_reference(tmp_path):
-    """f3: a demonstration directory written by the REFERENCE's `data.serialize.save` (its `huggingface_utils` over the real
-    `datasets` package; `jsonpickle` through the names-only shim) is read by `imitation_b200.data.serialize.load`, and a
-    directory written by this repo's `save` is read by the reference's `load` -- same trajectories both ways."""
-    pytest.importorskip("datasets")
-    refimport.load()
-    from imitation.data import serialize as ref_serialize
-    from imitation.data import types as ref_types
-
-    from imitation_b200.data import serialize, types
-
-    rng = np.random.default_rng(3)
-    spec = [(6, True, [{"step": i} for i in range(6)]), (2, False, None), (4, True, [{} for _ in range(4)])]
-
-    def make(T, discrete):
-        out = []
-        for n, term, infos in spec:
-            out.append(T.TrajectoryWithRew(obs=rng.standard_normal((n + 1, 5)).astype(np.float32),
-                                           acts=rng.integers(0, 3, n) if discrete else rng.uniform(-1, 1, (n, 2)).astype(np.float32),
-                                           infos=None if infos is None else np.array(infos), terminal=term,
-                                           rews=rng.standard_normal(n).astype(np.float32)))
-        return out
-
-    def same(a, b):
-        assert len(a) == len(b)
-        for x, y in zip(a, b):
-            np.testing.assert_array_equal(np.asarray(x.obs, dtype=np.float32), np.asarray(y.obs, dtype=np.float32))
-            np.testing.assert_array_equal(np.asarray(x.acts), np.asarray(y.acts))
-            np.testing.assert_array_equal(np.asarray(x.rews, dtype=np.float32), np.asarray(y.rews, dtype=np.float32))
-            assert bool(x.terminal) == bool(y.terminal)
-            xi = [{}] * len(x.acts) if x.infos is None else list(x.infos)
-            yi = [{}] * len(y.acts) if y.infos is None else list(y.infos)
-            assert xi == yi
-
-    for discrete in (False, True):
-        theirs = make(ref_types, discrete)
-        ref_serialize.save(tmp_path / f"ref_{int(discrete)}", theirs)          # the reference writes ...
-        same(theirs, serialize.load_with_rewards(tmp_path / f"ref_{int(discrete)}"))  # ... this repo reads
-        ours = make(types, discrete)
-        serialize.save(tmp_path / f"ours_{int(discrete)}", ours)              # this repo writes ...
-        same(ours, ref_serialize.load_with_rewards(tmp_path / f"ours_{int(discrete)}"))  # ... the reference reads
-
-
-def test_host_side_rollout_helpers_agree_with_the_reference():
-    """f4: `rollout_stats` (with and without Monitor infos), `discounted_sum`, the sample-until predicates and
-    `flatten_trajectories_with_rew` of imitation_b200.data.rollout against the reference's own functions
-    (data/rollout.py:193-286, 509-621, 728-745) on the same random trajectories."""
-    refimport.load()
-    from imitation.data import rollout as ref_rollout
-    from imitation.data import types as ref_types
-
-    from imitation_b200.data import rollout, types
-
-    rng = np.random.default_rng(5)
-    lens = [4, 9, 1, 6, 6]
-
-    def make(T, monitor):
-        out = []
-        for k, n in enumerate(lens):
-            rews = rng.standard_normal(n).astype(np.float32)
-            infos = None
-            if monitor and k != 2:  # one trajectory without infos: it is skipped by the Monitor statistics
-                infos = np.array([{} for _ in range(n - 1)] + [{"episode": {"r": float(rews.sum()) + 0.5 * k, "l": n}}])
-            out.append(T.TrajectoryWithRew(obs=rng.standard_normal((n + 1, 3)).astype(np.float32), acts=rng.integers(0, 2, n),
-                                           infos=infos, terminal=bool(k % 2), rews=rews))
-        return out
-
-    for monitor in (False, True):
-        state = rng.bit_generator.state
-        theirs = make(ref_types, monitor)
-        rng.bit_generator.state = state
-        ours = make(types, monitor)
-        want, got = ref_rollout.rollout_stats(theirs), rollout.rollout_stats(ours)
-        assert set(got) == set(want) and ("monitor_return_mean" in want) == monitor
-        for k in want:
-            assert got[k] == want[k] and type(got[k]) is type(want[k]), k
-        fw, fg = ref_rollout.flatten_trajectories_with_rew(theirs), rollout.flatten_trajectories_with_rew(ours)
-        for field in ("obs", "acts", "next_obs", "dones", "rews"):
-            np.testing.assert_array_equal(getattr(fg, field), getattr(fw, field), err_msg=field)
-        for kw in (dict(min_timesteps=20), dict(min_episodes=5), dict(min_timesteps=27, min_episodes=2), dict(min_episodes=6)):
-            assert rollout.make_sample_until(**kw)(ours) == ref_rollout.make_sample_until(**kw)(theirs), kw
-    for kw in (dict(), dict(min_timesteps=0), dict(min_episodes=-1)):
-        with pytest.raises(ValueError) as e1:
-            ref_rollout.make_sample_until(**kw)
-        with pytest.raises(ValueError) as e2:
-            rollout.make_sample_until(**kw)
-        assert str(e1.value) == str(e2.value)
-    arr = rng.standard_normal((7, 3))
-    for gamma in (1.0, 0.9):
-        np.testing.assert_allclose(rollout.discounted_sum(arr, gamma), ref_rollout.discounted_sum(arr, gamma), rtol=1e-12)
-        np.testing.assert_allclose(rollout.discounted_sum(arr[:, 0], gamma), ref_rollout.discounted_sum(arr[:, 0], gamma), rtol=1e-12)
-
-
-def test_fixed_horizon_check_agrees_with_the_reference():
-    """a21: BaseImitationAlgorithm._check_fixed_horizon (algorithms/base.py:69-108): same accept / reject decisions, same
-    remembered horizon and the same error text as the reference's class over sequences of episode lengths."""
-    refimport.load()
-    from imitation.algorithms import base as ref_base
-
-    from imitation_b200.algorithms import base
-
-    class Ours(base.BaseImitationAlgorithm):
-        pass
-
-    class Theirs(ref_base.BaseImitationAlgorithm):
-        pass
-
-    scripts = [[[5, 5], [5], [], [6]], [[3], [3, 3, 4]], [[], [7], [7, 7], [7]], [[2, 9]]]
-    for allow in (False, True):
-        for script in scripts:
-            a, b = Ours(allow_variable_horizon=allow), Theirs(allow_variable_horizon=allow)
-            for horizons in script:
-                errs = []
-                for algo in (a, b):
-                    try:
-                        algo._check_fixed_horizon(horizons)
-                        errs.append(None)
-                    except ValueError as e:
-                        errs.append(str(e))
-                assert (errs[0] is None) == (errs[1] is None), (allow, script, horizons)
-                if errs[0] is not None:
-                    assert errs[0] == errs[1]
-                    break
-                assert a._horizon == b._horizon
-
-
-def test_trajectory_and_transition_validation_agrees_with_the_reference():
-    """data/types.py:61-330: the same inputs are rejected with the same messages by this repo's Trajectory / TrajectoryWithRew /
-    Transitions and by the reference's."""
-    refimport.load()
-    from imitation.data import types as R
-
-    from imitation_b200.data import types as M
-
-    z = np.zeros
-    traj = {"len": dict(obs=z((3, 2)), acts=z(3), infos=None, terminal=True),
-            "infos": dict(obs=z((4, 2)), acts=z(3), infos=np.array([{}] * 2), terminal=True),
-            "empty": dict(obs=z((1, 2)), acts=z(0), infos=None, terminal=True)}
-    rews = {"shape": z((3, 1), np.float32), "dtype": z(3, np.int64)}
-    ok = dict(obs=z((3, 2)), acts=z(3), infos=np.array([{}] * 3), next_obs=z((3, 2)), dones=z(3, bool))
-    trans = {"next_obs": {**ok, "next_obs": z((3, 3))}, "dones_dtype": {**ok, "dones": z(3)},
-             "dones_shape": {**ok, "dones": z((3, 1), bool)}, "acts": {**ok, "acts": z(2)}, "infos": {**ok, "infos": np.array([{}] * 2)}}
-
-    def message(fn):
-        with pytest.raises(ValueError) as e:
-            fn()
-        return str(e.value)
-
-    for name, kw in traj.items():
-        assert message(lambda: M.Trajectory(**kw)) == message(lambda: R.Trajectory(**kw)), name
-    for name, r in rews.items():
-        kw = dict(obs=z((4, 2)), acts=z(3), infos=None, terminal=True, rews=r)
-        assert message(lambda: M.TrajectoryWithRew(**kw)) == message(lambda: R.TrajectoryWithRew(**kw)), name
-    for name, kw in trans.items():
-        assert message(lambda: M.Transitions(**kw)) == message(lambda: R.Transitions(**kw)), name
-    assert len(M.Transitions(**ok)) == len(R.Transitions(**ok)) == 3
-
-
-def test_comparison_schedule_helpers_agree_with_the_reference():
-    """f1: the per-iteration comparison counts of PreferenceComparisons.train (preference_comparisons.py:1622-1636) --
-    `util.oric` rounding of the query-schedule shares -- and the named query schedules (:1465-1479)."""
-    refimport.load()
-    from imitation.algorithms import preference_comparisons as ref_pc
-    from imitation.util import util as ref_util
-
-    from imitation_b200.algorithms import preference_comparisons as pc
-
-    rng = np.random.default_rng(0)
-    for _ in range(500):
-        n, total = int(rng.integers(1, 12)), int(rng.integers(0, 300))
-        v = rng.random(n) + 1e-3
-        x = v / v.sum() * total
-        np.testing.assert_array_equal(pc._round_keep_sum(x), ref_util.oric(x))
-    for n in (None, 1, 5):  # seeds handed to samplers / DataLoaders come from the caller's generator the same way
-        assert pc.make_seeds(np.random.default_rng(9), n) == ref_util.make_seeds(np.random.default_rng(9), n)
-    assert set(pc.QUERY_SCHEDULES) == set(ref_pc.QUERY_SCHEDULES)
-    for name, fn in pc.QUERY_SCHEDULES.items():
-        for t in np.linspace(0, 1, 7):
-            assert fn(t) == ref_pc.QUERY_SCHEDULES[name](t), (name, t)
-    # the whole schedule of a run: initial comparisons + oric(shares), as PreferenceComparisons.train computes it
-    for name in pc.QUERY_SCHEDULES:
-        for total, iters, frac in ((500, 5, 0.1), (77, 3, 0.25), (1000, 12, 0.1)):
-            initial = int(total * frac)
-            vec = np.array([pc.QUERY_SCHEDULES[name](t) for t in np.linspace(0, 1, iters)])
-            ours = [initial] + [int(v) for v in pc._round_keep_sum(vec / vec.sum() * (total - initial))]
-            rvec = np.array([ref_pc.QUERY_SCHEDULES[name](t) for t in np.linspace(0, 1, iters)])
-            theirs = [initial] + ref_util.oric(rvec / rvec.sum() * (total - initial)).tolist()
-            assert ours == theirs and sum(ours) == total
-
-
-def test_reward_net_preprocess_and_registry_agree_with_the_reference():
-    """a8 / f4: `RewardNet.preprocess` (reward_nets.py:74-118: float conversion, one-hot Discrete actions) on CPU tensors and
-    the registered reward-loader names of rewards/serialize.py:230-260 against the reference's."""
-    refimport.load()
-    import gymnasium
-    import torch as th
-    from imitation.rewards import reward_nets as ref_rn
-    from imitation.rewards import serialize as ref_ser
-
-    from imitation_b200 import spaces
-    from imitation_b200.rewards import reward_nets, serialize
-
-    assert sorted(serialize.reward_registry.keys()) == sorted(ref_ser.reward_registry.keys())
-    rng = np.random.default_rng(0)
-    for discrete in (True, False):
-        theirs = ref_rn.BasicRewardNet(gymnasium.spaces.Box(-1, 1, (4,)),
-                                       gymnasium.spaces.Discrete(3) if discrete else gymnasium.spaces.Box(-1, 1, (2,)))
-        ours = reward_nets.BasicRewardNet(spaces.Box(-1, 1, (4,)), spaces.Discrete(3) if discrete else spaces.Box(-1, 1, (2,)))
-        obs, nobs = rng.standard_normal((6, 4)), rng.standard_normal((6, 4)).astype(np.float32)
-        acts = rng.integers(0, 3, 6) if discrete else rng.uniform(-1, 1, (6, 2))
-        done = rng.random(6) < 0.5
-        for a, b in zip(ours.preprocess(obs, acts, nobs, done), theirs.preprocess(obs, acts, nobs, done)):
-            assert a.dtype == b.dtype and th.equal(a, b)
-        assert {k: tuple(v.shape) for k, v in ours.state_dict().items()} == {k: tuple(v.shape) for k, v in theirs.state_dict().items()}
-
-
-def test_trajectory_dataset_and_preference_dataset_agree_with_the_reference(tmp_path):
-    """f1 host side: `TrajectoryDataset.sample` (preference_comparisons.py:99-124: shuffled selection with the caller's
-    generator), `PreferenceDataset` FIFO / pickling (:909-997) against the reference's classes for the same seeds."""
-    refimport.load()
-    from imitation.algorithms import preference_comparisons as ref_pc
-    from imitation.data import types as ref_types
-
-    from imitation_b200.algorithms import preference_comparisons as pc
-    from imitation_b200.data import types
-
-    lens = [5, 9, 3, 7, 7, 4, 11]
-
-    def make(T):
-        r = np.random.default_rng(1)
-        return [T.TrajectoryWithRew(obs=r.standard_normal((n + 1, 3)).astype(np.float32), acts=r.integers(0, 2, n), infos=None,
-                                    terminal=True, rews=r.standard_normal(n).astype(np.float32)) for n in lens]
-
-    theirs, ours = make(ref_types), make(types)
-    a, b = ref_pc.TrajectoryDataset(theirs, np.random.default_rng(7)), pc.TrajectoryDataset(ours, np.random.default_rng(7))
-    for steps in (10, 25, 46, 1):
-        ta, tb = a.sample(steps), b.sample(steps)
-        assert [len(t) for t in ta] == [len(t) for t in tb]
-        assert all(np.array_equal(x.obs, y.obs) for x, y in zip(ta, tb))
-    with pytest.raises(RuntimeError) as e1:
-        a.sample(100)
-    with pytest.raises(RuntimeError) as e2:
-        b.sample(100)
-    assert str(e1.value) == str(e2.value)
-    da, db = ref_pc.PreferenceDataset(max_size=3), pc.PreferenceDataset(max_size=3)
-    for d, f in ((da, theirs), (db, ours)):
-        d.push([(f[0], f[1]), (f[2], f[3])], np.array([1.0, 0.0], np.float32))
-        d.push([(f[4], f[5]), (f[6], f[0])], np.array([0.5, 1.0], np.float32))
-    assert len(da) == len(db) == 3
-    np.testing.assert_array_equal(da.preferences, db.preferences)
-    for i in range(3):
-        (xa, ya), pa = da[i]
-        (xb, yb), pb = db[i]
-        assert pa == pb and np.array_equal(xa.obs, xb.obs) and np.array_equal(ya.acts, yb.acts)
-    db.save(tmp_path / "prefs.pkl")
-    back = pc.PreferenceDataset.load(tmp_path / "prefs.pkl")
-    assert len(back) == 3 and np.array_equal(back.preferences, db.preferences) and back.max_size == 3
-    for bad in (np.array([1.0], np.float32), np.array([1.0, 0.0], np.float64)):
-        msgs = []
-        for d, f in ((da, theirs), (db, ours)):
-            with pytest.raises(ValueError) as e:
-                d.push([(f[0], f[1]), (f[2], f[3])], bad)
-            msgs.append(str(e.value))
-        assert msgs[0] == msgs[1]
-
-
-def test_running_norm_module_and_mode_helpers_agree_with_the_reference():
-    """a10: the torch-level `RunningNorm` module (util/networks.py:19-134; the API path and the policy's
-    NormalizeFeaturesExtractor use it on whatever device the tensors are on) is bit-identical to the reference's over a
-    sequence of training batches and in eval mode; `training()` / `evaluating()` context managers restore the mode."""
-    refimport.load()
-    import torch as th
-    from imitation.util import networks as ref_networks
-
-    from imitation_b200.util import networks
-
-    a, b = ref_networks.RunningNorm(5), networks.RunningNorm(5)
-    g = th.Generator().manual_seed(0)
-    for step in range(5):
-        x = th.randn(7 + step, 5, generator=g) * (1 + step) + step
-        assert th.equal(a(x), b(x))
-        assert int(a.count) == int(b.count) and th.equal(a.running_mean, b.running_mean) and th.equal(a.running_var, b.running_var)
-    for m in (a, b):
-        m.eval()
-    x = th.randn(3, 5, generator=g)
-    assert th.equal(a(x), b(x)) and int(a.count) == int(b.count) == 45
-    assert {k: v.dtype for k, v in a.state_dict().items()} == {k: v.dtype for k, v in b.state_dict().items()}
-    b.load_state_dict(a.state_dict())
-    for ctx, want in ((networks.training, True), (networks.evaluating, False)):
-        b.eval()
-        with ctx(b):
-            assert b.training is want
-        assert b.training is False
-        b.train()
-        with ctx(b):
-            assert b.training is want
-        assert b.training is True
-
-
-def test_preference_probability_and_loss_agree_with_the_reference():
-    """f1: `PreferenceModel.probability` (preference_comparisons.py:487-530: discounting, clipping at the threshold, noise
-    floor) and the cross-entropy / accuracy arithmetic of `CrossEntropyRewardLoss` (:1043-1090) on CPU tensors against the
-    reference's classes, for several (noise_prob, discount_factor, threshold) settings incl. clipped return differences."""
-    refimport.load()
-    import gymnasium
-    import torch as th
-    from imitation.algorithms import preference_comparisons as ref_pc
-    from imitation.rewards import reward_nets as ref_rn
-
-    from imitation_b200 import spaces
-    from imitation_b200.algorithms import preference_comparisons as pc
-    from imitation_b200.rewards import reward_nets
-
-    theirs_net = ref_rn.BasicRewardNet(gymnasium.spaces.Box(-1, 1, (4,)), gymnasium.spaces.Box(-1, 1, (2,)))
-    ours_net = reward_nets.BasicRewardNet(spaces.Box(-1, 1, (4,)), spaces.Box(-1, 1, (2,)))
-    g = th.Generator().manual_seed(0)
-    for noise, discount, threshold in ((0.0, 1.0, 50.0), (0.1, 0.95, 50.0), (0.3, 0.9, 2.0)):
-        a = ref_pc.PreferenceModel(theirs_net, noise_prob=noise, discount_factor=discount, threshold=threshold)
-        b = pc.PreferenceModel(ours_net, noise_prob=noise, discount_factor=discount, threshold=threshold)
-        for scale in (0.3, 3.0):
-            r1, r2 = th.randn(12, generator=g) * scale, th.randn(12, generator=g) * scale
-            pa, pb = a.probability(r1, r2), b.probability(r1, r2)
-            assert pa.shape == pb.shape == () and th.equal(pa, pb)
-        # a batch of pairs the way the fused path lays it out: [P, L] rewards, time on axis 1
-        R1, R2 = th.randn(9, 12, generator=g) * 2, th.randn(9, 12, generator=g) * 2
-        batch = b._probability(R1, R2, time_axis=1)
-        single = th.stack([a.probability(x, y) for x, y in zip(R1, R2)])
-        th.testing.assert_close(batch, single, rtol=1e-6, atol=1e-7)
-        prefs = (th.rand(9, generator=g) < 0.5).float()
-        want = th.nn.functional.binary_cross_entropy(single, prefs)
-        th.testing.assert_close(th.nn.functional.binary_cross_entropy(batch, prefs), want, rtol=1e-6, atol=1e-7)
-        assert ((batch > 0.5) == (prefs > 0.5)).float().mean() == ((single > 0.5) == (prefs > 0.5)).float().mean()
+    assert common.__file__ == os.path.join(refimport.REF_SRC, "imitation", "algorithms", "adversarial", "common.py")

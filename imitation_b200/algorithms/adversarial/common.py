@@ -36,7 +36,7 @@ STAT_KEYS = ("disc_loss", "disc_acc", "disc_acc_expert", "disc_acc_gen", "disc_e
 def compute_train_stats(disc_logits_expert_is_high: th.Tensor, labels_expert_is_one: th.Tensor,
                         disc_loss: th.Tensor) -> Mapping[str, float]:
     """Torch restatement of common.py:27-92 for the generic (non-fused optimiser) path; the fused
-    path computes the same nine numbers inside the kernels (csrc/imb_disc.cu:k_disc_adam)."""
+    path computes the same nine numbers inside the kernels (csrc/imb_disc.cu:write_train_stats)."""
     with th.no_grad():
         logits, labels = disc_logits_expert_is_high, labels_expert_is_one
         pred_gen, true_gen = logits < 0, labels == 0

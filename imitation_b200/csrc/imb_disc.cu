@@ -1,23 +1,30 @@
 // imb_disc.cu -- stage 3 of the GAIL/AIRL round: the discriminator update, fused.
 //
-// Replaces (reference, /root/reference/src/imitation): rewards/reward_nets.py:441-457
+// Replaces (reference, paths relative to imitation's src/imitation): rewards/reward_nets.py:441-457
 // (BasicRewardNet.forward), :701-736 (ShapedRewardNet.forward), util/networks.py:79-134
 // (RunningNorm), algorithms/adversarial/common.py:353-372 (BCE-with-logits, backward, Adam)
 // and :27-92 (compute_train_stats).
 //
-// Kernel plan (no spinning grid barriers -- every dependency is a kernel boundary or the
+// Kernels (no spinning grid barriers -- every dependency is a kernel boundary or the
 // "last block done" ticket, so a bug cannot hang the GPU):
-//   k_norm_stats   per-chunk (n, mean, M2) per input feature; last CTA Chan-merges the chunks in
-//                  fixed order into the running stats (RunningNorm.update_stats).
-//   k_disc_fwdbwd  persistent CTAs over 128-row tiles of the feature-major batch.  The tile is
-//                  staged [feature][row] into shared memory by cp.async.bulk (TMA unit) with a
-//                  2-stage mbarrier pipeline.  Phase A (thread per row): normalise, MLP forward,
-//                  BCE-with-logits, backward to dL/dz per layer, activations to smem tiles.
-//                  Phase B (warps split output columns): the three weight-gradient contractions
-//                  dW = D^T . Act over the tile, accumulated in shared memory across tiles.
-//                  Weights (<34 KB) stay in shared memory; activations never touch HBM.
-//   k_disc_reduce  warp-per-parameter deterministic sum of the per-CTA partials.
-//   k_disc_adam    torch.optim.Adam step + the 9 train statistics.
+//   k_norm_stats        RunningNorm.update_stats for a list of up to three jobs (one normaliser each;
+//                       blockIdx.y = job): per-chunk (mean, M2) per input feature, then the last CTA
+//                       Chan-merges each job's chunks in a fixed order and folds the jobs into their
+//                       running statistics in job order -- or, for a one-job launch, appends the batch
+//                       moments to a deferred slot list.
+//   k_norm_fold         folds deferred slots into the running statistics, in order.
+//   k_disc_fwdbwd<R>    fp32-FFMA forward / BCE / backward: persistent CTAs over R-row tiles of the
+//                       feature-major batch staged by cp.async.bulk, tiled contractions of
+//                       imb_tile.cuh; one partial [gradient | statistics] row per CTA.
+//   k_disc_fwdbwd_tc    the same on the tcgen05 tensor cores (imb_disc_tc.cuh), used whenever the
+//                       network shape fits it.
+//   k_disc_reduce       warp-per-parameter deterministic sum of the per-CTA partials.
+//   k_disc_adam         torch.optim.Adam / AdamW step + the 9 train statistics.
+//   k_disc_reduce_adam  both in one launch: the last block to finish the reduction runs the step.
+//   k_pref_loss         preference comparisons: Boltzmann probability, cross entropy and its gradient.
+//   k_reward_fwd<H>     forward only (reward relabel / predict), thread per row.
+//   k_reward_norm_scan  NormalizedRewardNet.predict_processed over consecutive env steps.
+//   k_stats_publish, k_set_rows, k_set_meta, k_state_add: small bookkeeping kernels.
 #include <stdlib.h>
 
 #include "imb_common.cuh"
@@ -32,6 +39,7 @@ extern "C" const char* imb_last_error(void) { return g_imb_err; }
 namespace {
 
 constexpr int NORM_CHUNK = 512;       // rows per CTA in k_norm_stats
+constexpr int NORM_PS = 2 * IMB_MAX_DIN + 4;  // floats per chunk record of k_norm_stats: mean | M2 | n
 constexpr int MAXG = 296;             // max CTAs of k_disc_fwdbwd (2 per SM)
 
 // ---- workspace layout (floats) -----------------------------------------------------------------
@@ -41,7 +49,7 @@ struct WsLayout {
   int64_t meta;      // [16] ints: grid of the last fwdbwd launch, n rows, n_expert
   int64_t snap;      // [2*IMB_MAX_DIN] potential-norm stats after the first (next_obs) update
   int64_t ticket;    // [16] uint tickets
-  int64_t normpart;  // [MAXCHUNKS][2*IMB_MAX_DIN + 4]
+  int64_t normpart;  // [MAXCHUNKS][NORM_PS]
   int64_t partial;   // [MAXG][P + 16]
   int64_t total;
 };
@@ -61,7 +69,7 @@ inline WsLayout ws_layout(int P) {
   w.ticket = o;
   o += 32;
   w.normpart = o;
-  o += (int64_t)MAXCHUNKS * (2 * IMB_MAX_DIN + 4);
+  o += (int64_t)MAXCHUNKS * NORM_PS;
   w.partial = o;
   o += (int64_t)MAXG * part_stride(P);
   w.total = o;
@@ -69,194 +77,103 @@ inline WsLayout ws_layout(int P) {
 }
 
 // ---- RunningNorm statistics ----------------------------------------------------------------------
-struct NormLaunch {
+// One RunningNorm.update_stats per job.  A shaped net updates its potential's normaliser twice per training forward
+// (next_obs, then obs -- reward_nets.py:708-710), so two jobs may share one normaliser.
+struct NormJob {
   int din;
   short row[IMB_MAX_DIN];  // batch feature rows
+  float* rmv;              // running [mean | var] of the job's normaliser
+  int32_t* cnt;
+  float* snap;             // optional copy of the statistics after this job's fold
 };
-
-// One CTA per NORM_CHUNK rows; warp w handles features w, w+nw, ...: exact two-pass (mean, M2)
-// inside the chunk, then the last CTA to finish merges all chunks in index order (Chan et al.)
-// and folds the batch into the running statistics exactly as util/networks.py:111-134 does.
-__global__ void __launch_bounds__(256) k_norm_stats(NormLaunch L, const float* __restrict__ batch, int64_t ld,
-                                                    int64_t n, int chunk_rows, float* __restrict__ run_mean_var,
-                                                    int32_t* __restrict__ count, float* __restrict__ snap_out,
-                                                    float* __restrict__ part, unsigned int* __restrict__ ticket,
-                                                    float* __restrict__ defer = nullptr, int defer_cap = 0) {
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
-  const int64_t r0 = (int64_t)blockIdx.x * chunk_rows;
-  const int64_t r1 = min(n, r0 + (int64_t)chunk_rows);
-  const int cn = (int)(r1 - r0);
-  const int PS = 2 * IMB_MAX_DIN + 4;
-  float* my = part + (int64_t)blockIdx.x * PS;
-  for (int k = warp; k < L.din; k += nw) {
-    const float* src = batch + (int64_t)L.row[k] * ld + r0;
-    float s = 0.f;
-    for (int i = lane; i < cn; i += 32) s += src[i];
-    s = warp_sum(s);
-    const float mean = s / (float)cn;
-    float m2 = 0.f;
-    for (int i = lane; i < cn; i += 32) {
-      float dlt = src[i] - mean;
-      m2 = fmaf(dlt, dlt, m2);
-    }
-    m2 = warp_sum(m2);
-    if (lane == 0) {
-      my[k] = mean;
-      my[IMB_MAX_DIN + k] = m2;
-    }
-  }
-  if (threadIdx.x == 0) my[2 * IMB_MAX_DIN] = (float)cn;
-  __threadfence();
-  __shared__ bool is_last;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    unsigned int t = atomicAdd(ticket, 1u);
-    is_last = (t == gridDim.x - 1);
-  }
-  __syncthreads();
-  if (!is_last) return;
-  __threadfence();
-  // deferred mode: the batch moments go to the next free slot of `defer` ([0] = slot counter, slots of 2 * din + 1
-  // floats: mean | biased variance | n) instead of into the running statistics; k_norm_fold applies them later, in order
-  float* slot = nullptr;
-  if (defer) {
-    int k = (int)defer[0];
-    if (k >= defer_cap) k = defer_cap - 1;  // (host folds long before this; never overrun)
-    slot = defer + 4 + (int64_t)k * (2 * L.din + 1);
-  }
-  const int32_t old_count = defer ? 0 : *count;
-  // warp per feature: every lane Chan-merges its chunks (lane, lane + 32, ...) in index order, then the 32 lane
-  // results are merged by a fixed butterfly (deterministic; a single thread walking all chunks cost more than
-  // the statistics themselves once the chunks became small enough to fill the GPU)
-  for (int k = warp; k < L.din; k += nw) {
-    float na = 0.f, ma = 0.f, m2a = 0.f;
-    for (unsigned int c = lane; c < gridDim.x; c += 32) {
-      const float* p = part + (int64_t)c * PS;
-      const float nb = __ldcg(p + 2 * IMB_MAX_DIN), mb = __ldcg(p + k), m2b = __ldcg(p + IMB_MAX_DIN + k);
-      const float nt = na + nb;
-      const float dlt = mb - ma;
-      ma = ma + dlt * (nb / nt);
-      m2a = m2a + m2b + dlt * dlt * (na * nb / nt);
-      na = nt;
-    }
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const float nb = __shfl_xor_sync(0xffffffffu, na, o), mb = __shfl_xor_sync(0xffffffffu, ma, o),
-                  m2b = __shfl_xor_sync(0xffffffffu, m2a, o);
-      // merge (lower lane, higher lane) in that order on both sides so the pair agrees bit for bit
-      const bool lowme = (lane & o) == 0;
-      const float n1 = lowme ? na : nb, m1 = lowme ? ma : mb, q1 = lowme ? m2a : m2b;
-      const float n2 = lowme ? nb : na, m2v = lowme ? mb : ma, q2 = lowme ? m2b : m2a;
-      const float nt = n1 + n2;
-      if (nt > 0.f) {
-        const float dlt = m2v - m1;
-        ma = m1 + dlt * (n2 / nt);
-        m2a = q1 + q2 + dlt * dlt * (n1 * n2 / nt);
-      }
-      na = nt;
-    }
-    if (lane == 0 && slot) {
-      slot[k] = ma;
-      slot[L.din + k] = m2a / na;
-    } else if (lane == 0) {
-      const float b_mean = ma, b_var = m2a / na, b_n = na;
-      float mean = run_mean_var[k], var = run_mean_var[L.din + k];
-      const float cnt = (float)old_count;
-      const float tot = cnt + b_n;
-      const float delta = b_mean - mean;
-      mean += delta * b_n / tot;
-      var *= cnt;
-      var += b_var * b_n;
-      var += delta * delta * cnt * b_n / tot;
-      var /= tot;
-      run_mean_var[k] = mean;
-      run_mean_var[L.din + k] = var;
-      if (snap_out) {
-        snap_out[k] = mean;
-        snap_out[L.din + k] = var;
-      }
-    }
-  }
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    if (slot) {
-      slot[2 * L.din] = (float)n;
-      defer[0] += 1.0f;
-    } else {
-      *count = old_count + (int32_t)n;
-    }
-    *ticket = 0u;  // re-arm for the next launch
-  }
-}
-
-// fold the deferred batch moments into the running statistics, slot by slot, with RunningNorm.update_stats'
-// arithmetic (util/networks.py:121-134) -- the same expressions as the in-kernel fold of k_norm_stats
-__global__ void k_norm_fold(int din, float* __restrict__ defer, float* __restrict__ run_mean_var,
-                            int32_t* __restrict__ count, int k_fixed) {
-  const int K = k_fixed > 0 ? k_fixed : (int)defer[0];
-  const int k = threadIdx.x;
-  int32_t cnt_i = *count;
-  if (k < din) {
-    float mean = run_mean_var[k], var = run_mean_var[din + k];
-    int32_t c = cnt_i;
-    for (int sidx = 0; sidx < K; ++sidx) {
-      const float* slot = defer + 4 + (int64_t)sidx * (2 * din + 1);
-      const float b_mean = slot[k], b_var = slot[din + k], b_n = slot[2 * din];
-      const float cnt = (float)c;
-      const float tot = cnt + b_n;
-      const float delta = b_mean - mean;
-      mean += delta * b_n / tot;
-      var *= cnt;
-      var += b_var * b_n;
-      var += delta * delta * cnt * b_n / tot;
-      var /= tot;
-      c += (int32_t)b_n;
-    }
-    run_mean_var[k] = mean;
-    run_mean_var[din + k] = var;
-  }
-  __syncthreads();
-  if (k == 0) {
-    for (int sidx = 0; sidx < K; ++sidx) cnt_i += (int32_t)defer[4 + (int64_t)sidx * (2 * din + 1) + 2 * din];
-    *count = cnt_i;
-    if (k_fixed <= 0) defer[0] = 0.f;
-  }
-}
-
-// Several RunningNorm updates in ONE launch (AIRL: the base net's normaliser and the potential's, the latter updated twice:
-// first with next_obs, then with obs -- reward_nets.py:708-710).  blockIdx.y = job; every CTA computes the (mean, M2) of its
-// chunk of its job's rows; the last CTA of the whole grid Chan-merges each job's chunks and folds the jobs into their
-// running statistics IN JOB ORDER (two jobs may share a normaliser; `snap` receives the statistics right after a job's fold).
 struct NormJobs {
   int njobs;
-  NormLaunch job[3];
-  float* rmv[3];       // running [mean | var] of the job's normaliser
-  int32_t* cnt[3];
-  float* snap[3];      // optional copy of the statistics after this job's fold
+  NormJob job[3];
 };
-__global__ void __launch_bounds__(256) k_norm_stats_multi(NormJobs J, const float* __restrict__ batch, int64_t ld, int64_t n,
-                                                          int chunk_rows, float* __restrict__ part,
-                                                          unsigned int* __restrict__ ticket) {
+
+// exact two-pass (mean, M2) of the cn values at src, by one warp
+__device__ __forceinline__ void chunk_moments(const float* src, int cn, int lane, float& mean, float& m2) {
+  float s = 0.f;
+  for (int i = lane; i < cn; i += 32) s += src[i];
+  s = warp_sum(s);
+  mean = s / (float)cn;
+  m2 = 0.f;
+  for (int i = lane; i < cn; i += 32) {
+    float dlt = src[i] - mean;
+    m2 = fmaf(dlt, dlt, m2);
+  }
+  m2 = warp_sum(m2);
+}
+
+// Chan et al. merge of feature k over the nchunks chunk records at `part`, by one warp: every lane merges its chunks
+// (lane, lane + 32, ...) in index order, then the 32 lane results are merged by a fixed butterfly (deterministic; a
+// single thread walking all chunks cost more than the statistics themselves once the chunks became small enough to fill
+// the GPU).  Every lane ends with (n, mean, M2) of the whole batch.
+__device__ __forceinline__ void chan_merge_chunks(const float* part, int nchunks, int k, int lane, float& na, float& ma,
+                                                  float& m2a) {
+  na = 0.f;
+  ma = 0.f;
+  m2a = 0.f;
+  for (int c = lane; c < nchunks; c += 32) {
+    const float* p = part + (int64_t)c * NORM_PS;
+    const float nb = __ldcg(p + 2 * IMB_MAX_DIN), mb = __ldcg(p + k), m2b = __ldcg(p + IMB_MAX_DIN + k);
+    const float nt = na + nb;
+    const float dlt = mb - ma;
+    ma = ma + dlt * (nb / nt);
+    m2a = m2a + m2b + dlt * dlt * (na * nb / nt);
+    na = nt;
+  }
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const float nb = __shfl_xor_sync(0xffffffffu, na, o), mb = __shfl_xor_sync(0xffffffffu, ma, o),
+                m2b = __shfl_xor_sync(0xffffffffu, m2a, o);
+    // merge (lower lane, higher lane) in that order on both sides so the pair agrees bit for bit
+    const bool lowme = (lane & o) == 0;
+    const float n1 = lowme ? na : nb, m1 = lowme ? ma : mb, q1 = lowme ? m2a : m2b;
+    const float n2 = lowme ? nb : na, m2v = lowme ? mb : ma, q2 = lowme ? m2b : m2a;
+    const float nt = n1 + n2;
+    if (nt > 0.f) {
+      const float dlt = m2v - m1;
+      ma = m1 + dlt * (n2 / nt);
+      m2a = q1 + q2 + dlt * dlt * (n1 * n2 / nt);
+    }
+    na = nt;
+  }
+}
+
+// fold batch moments (b_mean, biased b_var, b_n rows) into running statistics over cnt earlier rows with
+// RunningNorm.update_stats' arithmetic (util/networks.py:121-134).  nvcc contracts `var * cnt + b_var * b_n` per call
+// site: fma(b_var, b_n, var * cnt) in k_norm_stats, fma(var, cnt, b_var * b_n) in k_norm_fold, so an immediate and a
+// deferred fold of the same batch can differ in the last bit of the variance.
+__device__ __forceinline__ void fold_moments(float& mean, float& var, float cnt, float b_mean, float b_var, float b_n) {
+  const float tot = cnt + b_n;
+  const float delta = b_mean - mean;
+  mean += delta * b_n / tot;
+  var *= cnt;
+  var += b_var * b_n;
+  var += delta * delta * cnt * b_n / tot;
+  var /= tot;
+}
+
+// One CTA per chunk_rows rows of job blockIdx.y; warp w handles features w, w+nw, ...  The last CTA of the grid merges
+// each job's chunks and folds the jobs into their running statistics in job order (a later job may read what an earlier
+// one wrote).  Deferred mode, for one-job launches only: the batch moments go to the next free slot of `defer` ([0] =
+// slot counter, slots of 2 * din + 1 floats: mean | biased variance | n) instead of into the running statistics;
+// k_norm_fold applies them later, in order.
+__global__ void __launch_bounds__(256) k_norm_stats(NormJobs J, const float* __restrict__ batch, int64_t ld, int64_t n,
+                                                    int chunk_rows, float* __restrict__ part,
+                                                    unsigned int* __restrict__ ticket, float* __restrict__ defer,
+                                                    int defer_cap) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
-  const int jb = blockIdx.y, nchunks = gridDim.x;
-  const NormLaunch& L = J.job[jb];
+  const int nchunks = gridDim.x;
+  const NormJob& L = J.job[blockIdx.y];
   const int64_t r0 = (int64_t)blockIdx.x * chunk_rows;
   const int64_t r1 = min(n, r0 + (int64_t)chunk_rows);
   const int cn = (int)(r1 - r0);
-  const int PS = 2 * IMB_MAX_DIN + 4;
-  float* my = part + ((int64_t)jb * nchunks + blockIdx.x) * PS;
+  float* my = part + ((int64_t)blockIdx.y * nchunks + blockIdx.x) * NORM_PS;
   for (int k = warp; k < L.din; k += nw) {
-    const float* src = batch + (int64_t)L.row[k] * ld + r0;
-    float s = 0.f;
-    for (int i = lane; i < cn; i += 32) s += src[i];
-    s = warp_sum(s);
-    const float mean = s / (float)cn;
-    float m2 = 0.f;
-    for (int i = lane; i < cn; i += 32) {
-      float dlt = src[i] - mean;
-      m2 = fmaf(dlt, dlt, m2);
-    }
-    m2 = warp_sum(m2);
+    float mean, m2;
+    chunk_moments(batch + (int64_t)L.row[k] * ld + r0, cn, lane, mean, m2);
     if (lane == 0) {
       my[k] = mean;
       my[IMB_MAX_DIN + k] = m2;
@@ -273,60 +190,70 @@ __global__ void __launch_bounds__(256) k_norm_stats_multi(NormJobs J, const floa
   __syncthreads();
   if (!is_last) return;
   __threadfence();
-  for (int job = 0; job < J.njobs; ++job) {  // folds in job order (a later job may read what an earlier one wrote)
-    const NormLaunch& Lj = J.job[job];
-    const int32_t old_count = *J.cnt[job];
-    float* run_mean_var = J.rmv[job];
+  float* slot = nullptr;
+  if (defer) {
+    int k = (int)defer[0];
+    if (k >= defer_cap) k = defer_cap - 1;  // (host folds long before this; never overrun)
+    slot = defer + 4 + (int64_t)k * (2 * J.job[0].din + 1);
+  }
+  for (int job = 0; job < J.njobs; ++job) {
+    const NormJob& Lj = J.job[job];
+    const int32_t old_count = slot ? 0 : *Lj.cnt;
     for (int k = warp; k < Lj.din; k += nw) {
-      float na = 0.f, ma = 0.f, m2a = 0.f;
-      for (int c = lane; c < nchunks; c += 32) {
-        const float* p = part + ((int64_t)job * nchunks + c) * PS;
-        const float nb = __ldcg(p + 2 * IMB_MAX_DIN), mb = __ldcg(p + k), m2b = __ldcg(p + IMB_MAX_DIN + k);
-        const float nt = na + nb;
-        const float dlt = mb - ma;
-        ma = ma + dlt * (nb / nt);
-        m2a = m2a + m2b + dlt * dlt * (na * nb / nt);
-        na = nt;
-      }
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const float nb = __shfl_xor_sync(0xffffffffu, na, o), mb = __shfl_xor_sync(0xffffffffu, ma, o),
-                    m2b = __shfl_xor_sync(0xffffffffu, m2a, o);
-        const bool lowme = (lane & o) == 0;
-        const float n1 = lowme ? na : nb, m1 = lowme ? ma : mb, q1 = lowme ? m2a : m2b;
-        const float n2 = lowme ? nb : na, m2v = lowme ? mb : ma, q2 = lowme ? m2b : m2a;
-        const float nt = n1 + n2;
-        if (nt > 0.f) {
-          const float dlt = m2v - m1;
-          ma = m1 + dlt * (n2 / nt);
-          m2a = q1 + q2 + dlt * dlt * (n1 * n2 / nt);
-        }
-        na = nt;
-      }
-      if (lane == 0) {
-        const float b_mean = ma, b_var = m2a / na, b_n = na;
-        float mean = run_mean_var[k], var = run_mean_var[Lj.din + k];
-        const float cnt = (float)old_count;
-        const float tot = cnt + b_n;
-        const float delta = b_mean - mean;
-        mean += delta * b_n / tot;
-        var *= cnt;
-        var += b_var * b_n;
-        var += delta * delta * cnt * b_n / tot;
-        var /= tot;
-        run_mean_var[k] = mean;
-        run_mean_var[Lj.din + k] = var;
-        if (J.snap[job]) {
-          J.snap[job][k] = mean;
-          J.snap[job][Lj.din + k] = var;
+      float na, ma, m2a;
+      chan_merge_chunks(part + (int64_t)job * nchunks * NORM_PS, nchunks, k, lane, na, ma, m2a);
+      if (lane == 0 && slot) {
+        slot[k] = ma;
+        slot[Lj.din + k] = m2a / na;
+      } else if (lane == 0) {
+        float mean = Lj.rmv[k], var = Lj.rmv[Lj.din + k];
+        fold_moments(mean, var, (float)old_count, ma, m2a / na, na);
+        Lj.rmv[k] = mean;
+        Lj.rmv[Lj.din + k] = var;
+        if (Lj.snap) {
+          Lj.snap[k] = mean;
+          Lj.snap[Lj.din + k] = var;
         }
       }
     }
     __syncthreads();
-    if (threadIdx.x == 0) *J.cnt[job] = old_count + (int32_t)n;
+    if (threadIdx.x == 0) {
+      if (slot) {
+        slot[2 * Lj.din] = (float)n;
+        defer[0] += 1.0f;
+      } else {
+        *Lj.cnt = old_count + (int32_t)n;
+      }
+    }
     __syncthreads();  // the next job may fold into the same normaliser: count and statistics are in place
   }
   if (threadIdx.x == 0) *ticket = 0u;  // re-arm for the next launch
+}
+
+// fold the deferred batch moments into the running statistics, slot by slot
+__global__ void k_norm_fold(int din, float* __restrict__ defer, float* __restrict__ run_mean_var,
+                            int32_t* __restrict__ count, int k_fixed) {
+  const int K = k_fixed > 0 ? k_fixed : (int)defer[0];
+  const int k = threadIdx.x;
+  int32_t cnt_i = *count;
+  if (k < din) {
+    float mean = run_mean_var[k], var = run_mean_var[din + k];
+    int32_t c = cnt_i;
+    for (int sidx = 0; sidx < K; ++sidx) {
+      const float* slot = defer + 4 + (int64_t)sidx * (2 * din + 1);
+      const float b_n = slot[2 * din];
+      fold_moments(mean, var, (float)c, slot[k], slot[din + k], b_n);
+      c += (int32_t)b_n;
+    }
+    run_mean_var[k] = mean;
+    run_mean_var[din + k] = var;
+  }
+  __syncthreads();
+  if (k == 0) {
+    for (int sidx = 0; sidx < K; ++sidx) cnt_i += (int32_t)defer[4 + (int64_t)sidx * (2 * din + 1) + 2 * din];
+    *count = cnt_i;
+    if (k_fixed <= 0) defer[0] = 0.f;
+  }
 }
 
 // ---- the fused forward / BCE / backward kernel (tiled-GEMM form, see imb_tile.cuh) ------------------
@@ -705,12 +632,10 @@ __global__ void __launch_bounds__(R, 256 / R) k_disc_fwdbwd(const DiscLaunch L, 
 namespace {
 
 // ---- deterministic reduction of the per-CTA partials -----------------------------------------
-// warp per parameter (and per statistic): lanes stride over the G partial rows, shuffle-reduce.
-__global__ void __launch_bounds__(256) k_disc_reduce(int P, int G, const float* __restrict__ partial,
-                                                    float* __restrict__ gacc, float* __restrict__ stats,
-                                                    float* __restrict__ grad_out_flat) {
-  // (the Adam step number is read by k_disc_adam from the device counter block; the increment is
-  //  committed by a single thread there AFTER every block has read it -- see k_disc_adam)
+// warp per parameter (and per statistic): lanes stride over the G partial rows, shuffle-reduce.  Parameter sums are
+// added to the gradient accumulator (and copied to grad_out_flat if given); statistic sums replace the previous ones.
+__device__ __forceinline__ void reduce_partials(int P, int G, const float* __restrict__ partial, float* __restrict__ gacc,
+                                                float* __restrict__ stats, float* __restrict__ grad_out_flat) {
   const int gw = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   const int nwarps = (gridDim.x * blockDim.x) >> 5;
@@ -731,6 +656,12 @@ __global__ void __launch_bounds__(256) k_disc_reduce(int P, int G, const float* 
   }
 }
 
+__global__ void __launch_bounds__(256) k_disc_reduce(int P, int G, const float* __restrict__ partial,
+                                                    float* __restrict__ gacc, float* __restrict__ stats,
+                                                    float* __restrict__ grad_out_flat) {
+  reduce_partials(P, G, partial, gacc, stats, grad_out_flat);
+}
+
 // beta^n for an integer step count by repeated squaring (pow(double, double) costs microseconds on one thread)
 __device__ __forceinline__ double dpowi(double b, int64_t n) {
   double r = 1.0;
@@ -742,14 +673,11 @@ __device__ __forceinline__ double dpowi(double b, int64_t n) {
   return r;
 }
 
-// single block: every thread reads the step counter before thread 0 commits the increment (no race,
-// no extra launch); P <= ~8.5k parameters = a handful of iterations per thread.
-__global__ void __launch_bounds__(1024) k_disc_adam(int P, imb_adam opt, float* __restrict__ params,
-                                                  float* __restrict__ m, float* __restrict__ v,
-                                                  const float* __restrict__ grad, float grad_div,
-                                                  const float* __restrict__ stats, const int* __restrict__ meta,
-                                                  int64_t* __restrict__ step_io,
-                                                  float* __restrict__ stats_out) {
+// torch.optim.Adam / AdamW step by one block: thread 0 computes the bias corrections and commits the step counter, then
+// the block strides over the P elements.  grad is read through L2: in k_disc_reduce_adam other blocks wrote it.
+__device__ __forceinline__ void adam_step(int P, const imb_adam& opt, float* __restrict__ params, float* __restrict__ m,
+                                          float* __restrict__ v, const float* grad, float grad_div,
+                                          int64_t* __restrict__ step_io) {
   // bias corrections in double like torch's Python-scalar arithmetic (torch/optim/adam.py)
   __shared__ float s_bc[2];
   if (threadIdx.x == 0) {
@@ -763,7 +691,7 @@ __global__ void __launch_bounds__(1024) k_disc_adam(int P, imb_adam opt, float* 
   __syncthreads();
   const float step_size = s_bc[0], bc2_sqrt = s_bc[1];
   for (int i = threadIdx.x; i < P; i += blockDim.x) {
-    const float g = grad[i] / grad_div;
+    const float g = __ldcg(grad + i) / grad_div;
     const float mi = m[i] + (g - m[i]) * (1.0f - opt.beta1);        // torch: exp_avg.lerp_(grad, 1-beta1)
     const float vi = v[i] * opt.beta2 + (1.0f - opt.beta2) * g * g;  // exp_avg_sq.mul_(b2).addcmul_(g,g,1-b2)
     m[i] = mi;
@@ -772,20 +700,36 @@ __global__ void __launch_bounds__(1024) k_disc_adam(int P, imb_adam opt, float* 
     const float pw = opt.weight_decay > 0.f ? params[i] * (1.0f - opt.lr * opt.weight_decay) : params[i];  // AdamW
     params[i] = pw - step_size * (mi / denom);
   }
-  if (blockIdx.x == 0 && threadIdx.x == 0 && stats_out) {
-    const float n = (float)meta[1], n_exp = (float)meta[2], n_gen = n - n_exp;
-    const float loss_sum = stats[0], ent_sum = stats[1], c_exp = stats[2], c_gen = stats[3], c_pred = stats[4];
-    const float nanv = __int_as_float(0x7fc00000);
-    stats_out[0] = loss_sum * reinterpret_cast<const float*>(meta)[3];                 // disc_loss (scaled minibatch mean)
-    stats_out[1] = n > 0 ? (c_exp + c_gen) / n : nanv;         // disc_acc
-    stats_out[2] = n_exp >= 1 ? c_exp / n_exp : nanv;          // disc_acc_expert
-    stats_out[3] = c_gen / fmaxf(1.f, n_gen);                  // disc_acc_gen
-    stats_out[4] = n > 0 ? ent_sum / n : nanv;                 // disc_entropy
-    stats_out[5] = n > 0 ? n_exp / n : nanv;                   // disc_proportion_expert_true
-    stats_out[6] = n > 0 ? c_pred / n : nanv;                  // disc_proportion_expert_pred
-    stats_out[7] = n_exp;
-    stats_out[8] = n_gen;
-  }
+}
+
+// the nine statistics of compute_train_stats (common.py:27-92), by one thread, from the reduced sums of the last
+// minibatch and its launch record (meta: n rows, n_expert, loss scale).  stats is read through L2: in
+// k_disc_reduce_adam other blocks wrote it.
+__device__ __forceinline__ void write_train_stats(const float* stats, const int* meta, float* stats_out) {
+  const float n = (float)meta[1], n_exp = (float)meta[2], n_gen = n - n_exp;
+  const float loss_sum = __ldcg(stats + 0), ent_sum = __ldcg(stats + 1), c_exp = __ldcg(stats + 2),
+              c_gen = __ldcg(stats + 3), c_pred = __ldcg(stats + 4);
+  const float nanv = __int_as_float(0x7fc00000);
+  stats_out[0] = loss_sum * reinterpret_cast<const float*>(meta)[3];  // disc_loss (scaled minibatch mean)
+  stats_out[1] = n > 0 ? (c_exp + c_gen) / n : nanv;                  // disc_acc
+  stats_out[2] = n_exp >= 1 ? c_exp / n_exp : nanv;                   // disc_acc_expert
+  stats_out[3] = c_gen / fmaxf(1.f, n_gen);                           // disc_acc_gen
+  stats_out[4] = n > 0 ? ent_sum / n : nanv;                          // disc_entropy
+  stats_out[5] = n > 0 ? n_exp / n : nanv;                            // disc_proportion_expert_true
+  stats_out[6] = n > 0 ? c_pred / n : nanv;                           // disc_proportion_expert_pred
+  stats_out[7] = n_exp;
+  stats_out[8] = n_gen;
+}
+
+// single block: P <= ~8.5k parameters = a handful of iterations per thread.
+__global__ void __launch_bounds__(1024) k_disc_adam(int P, imb_adam opt, float* __restrict__ params,
+                                                  float* __restrict__ m, float* __restrict__ v,
+                                                  const float* __restrict__ grad, float grad_div,
+                                                  const float* __restrict__ stats, const int* __restrict__ meta,
+                                                  int64_t* __restrict__ step_io,
+                                                  float* __restrict__ stats_out) {
+  adam_step(P, opt, params, m, v, grad, grad_div, step_io);
+  if (threadIdx.x == 0 && stats_out) write_train_stats(stats, meta, stats_out);
 }
 
 // reduce + Adam in one launch (the last minibatch of an update): every block reduces its share of the partials
@@ -797,22 +741,9 @@ __global__ void __launch_bounds__(256) k_disc_reduce_adam(int P, int G, const fl
                                                          const int* __restrict__ meta, int64_t* __restrict__ step_io,
                                                          float* __restrict__ stats_out,
                                                          unsigned int* __restrict__ ticket) {
-  const int gw = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int lane = threadIdx.x & 31;
-  const int nwarps = (gridDim.x * blockDim.x) >> 5;
-  const int64_t ps = part_stride(P);
-  for (int p = gw; p < P + 5; p += nwarps) {
-    float acc = 0.f;
-    for (int c = lane; c < G; c += 32) acc += partial[(int64_t)c * ps + p];
-    acc = warp_sum(acc);
-    if (lane == 0) {
-      if (p < P) gacc[p] += acc;
-      else stats[p - P] = acc;
-    }
-  }
+  reduce_partials(P, G, partial, gacc, stats, nullptr);
   __threadfence();
   __shared__ bool is_last;
-  __shared__ float s_bc[2];
   __syncthreads();
   if (threadIdx.x == 0) {
     const unsigned int t = atomicAdd(ticket, 1u);
@@ -821,42 +752,9 @@ __global__ void __launch_bounds__(256) k_disc_reduce_adam(int P, int G, const fl
   __syncthreads();
   if (!is_last) return;
   __threadfence();
-  if (threadIdx.x == 0) {
-    const int64_t step = *step_io + 1;
-    const double bc1d = 1.0 - dpowi((double)opt.beta1, step);
-    const double bc2d = 1.0 - dpowi((double)opt.beta2, step);
-    s_bc[0] = (float)((double)opt.lr / bc1d);
-    s_bc[1] = (float)sqrt(bc2d);
-    *step_io = step;
-    *ticket = 0u;  // re-arm for the next launch
-  }
-  __syncthreads();
-  const float step_size = s_bc[0], bc2_sqrt = s_bc[1];
-  for (int i = threadIdx.x; i < P; i += blockDim.x) {
-    const float g = __ldcg(gacc + i) / grad_div;
-    const float mi = m[i] + (g - m[i]) * (1.0f - opt.beta1);
-    const float vi = v[i] * opt.beta2 + (1.0f - opt.beta2) * g * g;
-    m[i] = mi;
-    v[i] = vi;
-    const float denom = sqrtf(vi) / bc2_sqrt + opt.eps;
-    const float pw = opt.weight_decay > 0.f ? params[i] * (1.0f - opt.lr * opt.weight_decay) : params[i];  // AdamW
-    params[i] = pw - step_size * (mi / denom);
-  }
-  if (threadIdx.x == 0 && stats_out) {
-    const float n = (float)meta[1], n_exp = (float)meta[2], n_gen = n - n_exp;
-    const float loss_sum = __ldcg(stats + 0), ent_sum = __ldcg(stats + 1), c_exp = __ldcg(stats + 2),
-                c_gen = __ldcg(stats + 3), c_pred = __ldcg(stats + 4);
-    const float nanv = __int_as_float(0x7fc00000);
-    stats_out[0] = loss_sum * reinterpret_cast<const float*>(meta)[3];
-    stats_out[1] = n > 0 ? (c_exp + c_gen) / n : nanv;
-    stats_out[2] = n_exp >= 1 ? c_exp / n_exp : nanv;
-    stats_out[3] = c_gen / fmaxf(1.f, n_gen);
-    stats_out[4] = n > 0 ? ent_sum / n : nanv;
-    stats_out[5] = n > 0 ? n_exp / n : nanv;
-    stats_out[6] = n > 0 ? c_pred / n : nanv;
-    stats_out[7] = n_exp;
-    stats_out[8] = n_gen;
-  }
+  if (threadIdx.x == 0) *ticket = 0u;  // re-arm for the next launch
+  adam_step(P, opt, params, m, v, gacc, grad_div, step_io);
+  if (threadIdx.x == 0 && stats_out) write_train_stats(stats, meta, stats_out);
 }
 
 // ---- preference comparisons: fragment returns -> Boltzmann probability -> cross entropy (+ its gradient) -------------
@@ -1039,13 +937,7 @@ __global__ void __launch_bounds__(1024) k_reward_norm_scan(float* __restrict__ r
     }
     __syncthreads();
     if (update) {
-      const float bvar = bc[1], bn = (float)E, c = (float)cnt, tot = c + bn;
-      const float delta = bmean - mean;
-      mean += delta * bn / tot;
-      var *= c;
-      var += bvar * bn;
-      var += delta * delta * c * bn / tot;
-      var /= tot;
+      fold_moments(mean, var, (float)cnt, bmean, bc[1], (float)E);
       cnt += (int32_t)E;
     }
     __syncthreads();
@@ -1091,90 +983,70 @@ inline int pick_H(const DiscLaunch& L) {
 
 extern "C" int64_t imb_disc_workspace_floats(const imb_disc_desc* d) { return ws_layout(d->n_params).total; }
 
-static int norm_launch(const imb_mlp& m, const short* rows, const float* batch, int64_t ld, int64_t n,
-                       float* norm_state, int32_t* norm_count, float* snap, float* ws, const WsLayout& w,
-                       cudaStream_t st) {
-  NormLaunch NL;
-  NL.din = m.din;
-  for (int k = 0; k < m.din; ++k) NL.row[k] = rows[k];
+// RunningNorm updates of the jobs in J from batch rows [0, n): one launch when the chunk table holds every job's chunks,
+// else one launch per job, in job order
+static int norm_stats(const NormJobs& J, const float* batch, int64_t ld, int64_t n, float* defer, int defer_cap,
+                      float* ws, const WsLayout& w, cudaStream_t st) {
   // chunk size: small enough to fill the GPU at the tuned batch sizes (16 384 rows -> 128 CTAs), larger for the
   // multi-million-row sweeps so the chunk table stays bounded
   const int chunk_rows = n <= (int64_t)128 * 2048 ? 128 : NORM_CHUNK;
   const int chunks = (int)((n + chunk_rows - 1) / chunk_rows);
   IMB_REQUIRE(chunks >= 1 && chunks <= MAXCHUNKS, "norm update: n=%lld out of range", (long long)n);
-  k_norm_stats<<<chunks, 256, 0, st>>>(NL, batch, ld, n, chunk_rows, norm_state + m.norm_off, norm_count + m.count_idx, snap,
-                                       ws + w.normpart, reinterpret_cast<unsigned int*>(ws + w.ticket));
-  IMB_CHECK_LAUNCH("k_norm_stats");
+  float* part = ws + w.normpart;
+  unsigned int* ticket = reinterpret_cast<unsigned int*>(ws + w.ticket);
+  if ((int64_t)chunks * J.njobs <= MAXCHUNKS) {
+    k_norm_stats<<<dim3(chunks, J.njobs), 256, 0, st>>>(J, batch, ld, n, chunk_rows, part, ticket, defer, defer_cap);
+    IMB_CHECK_LAUNCH("k_norm_stats");
+    return 0;
+  }
+  for (int j = 0; j < J.njobs; ++j) {
+    NormJobs one{};
+    one.njobs = 1;
+    one.job[0] = J.job[j];
+    k_norm_stats<<<chunks, 256, 0, st>>>(one, batch, ld, n, chunk_rows, part, ticket, defer, defer_cap);
+    IMB_CHECK_LAUNCH("k_norm_stats");
+  }
   return 0;
 }
 
 extern "C" int imb_disc_norm_update(const imb_disc_desc* d, const float* batch, int64_t ld, int64_t n,
                                     float* norm_state, int32_t* norm_count, float* ws, void* stream) {
-  cudaStream_t st = (cudaStream_t)stream;
   IMB_REQUIRE(n >= 1, "norm update needs n >= 1");
   const WsLayout w = ws_layout(d->n_params);
   DiscLaunch L;
   if (int rc = build_launch(d, norm_state, nullptr, L)) return rc;
-  short rows[IMB_MAX_DIN];
-  // shaped nets: all updates of one training forward in ONE launch (base normaliser; potential normaliser with next_obs,
-  // then with obs -- reference order, both on the same RunningNorm) when the chunk table has room for the jobs
+  // the base normaliser, then for a shaped net the potential's with next_obs and then with obs (reference order, both on
+  // the same RunningNorm; the Phi(s') pass of the forward reads the snapshot taken between the two)
+  NormJobs J{};
+  auto add = [&](const imb_mlp& m, int pass, float* snap) {
+    NormJob& j = J.job[J.njobs++];
+    j.din = m.din;
+    for (int k = 0; k < m.din; ++k) j.row[k] = L.stage_row[L.pass[pass].in_slot[k]];
+    j.rmv = norm_state + m.norm_off;
+    j.cnt = norm_count + m.count_idx;
+    j.snap = snap;
+  };
+  if (d->base.has_norm) add(d->base, 0, nullptr);
   if (d->shaped && d->potential.has_norm) {
-    const int chunk_rows = n <= (int64_t)128 * 2048 ? 128 : NORM_CHUNK;
-    const int chunks = (int)((n + chunk_rows - 1) / chunk_rows);
-    NormJobs J;
-    memset(&J, 0, sizeof(J));
-    int nj = 0;
-    auto add = [&](const imb_mlp& m, int pass, float* snap) {
-      J.job[nj].din = m.din;
-      for (int k = 0; k < m.din; ++k) J.job[nj].row[k] = L.stage_row[L.pass[pass].in_slot[k]];
-      J.rmv[nj] = norm_state + m.norm_off;
-      J.cnt[nj] = norm_count + m.count_idx;
-      J.snap[nj] = snap;
-      ++nj;
-    };
-    if (d->base.has_norm) add(d->base, 0, nullptr);
     add(d->potential, 1, ws + w.snap);
     add(d->potential, 2, nullptr);
-    J.njobs = nj;
-    if ((int64_t)chunks * nj <= MAXCHUNKS) {
-      k_norm_stats_multi<<<dim3(chunks, nj), 256, 0, st>>>(J, batch, ld, n, chunk_rows, ws + w.normpart,
-                                                           reinterpret_cast<unsigned int*>(ws + w.ticket));
-      IMB_CHECK_LAUNCH("k_norm_stats_multi");
-      return 0;
-    }
   }
-  if (d->base.has_norm) {
-    for (int k = 0; k < d->base.din; ++k) rows[k] = L.stage_row[L.pass[0].in_slot[k]];
-    if (int rc = norm_launch(d->base, rows, batch, ld, n, norm_state, norm_count, nullptr, ws, w, st)) return rc;
-  }
-  if (d->shaped && d->potential.has_norm) {
-    // reference order: Phi(next_state) first, then Phi(state); both update the same RunningNorm
-    for (int k = 0; k < d->potential.din; ++k) rows[k] = L.stage_row[L.pass[1].in_slot[k]];
-    if (int rc = norm_launch(d->potential, rows, batch, ld, n, norm_state, norm_count, ws + w.snap, ws, w, st))
-      return rc;
-    for (int k = 0; k < d->potential.din; ++k) rows[k] = L.stage_row[L.pass[2].in_slot[k]];
-    if (int rc = norm_launch(d->potential, rows, batch, ld, n, norm_state, norm_count, nullptr, ws, w, st)) return rc;
-  }
-  return 0;
+  if (J.njobs == 0) return 0;
+  return norm_stats(J, batch, ld, n, nullptr, 0, ws, w, (cudaStream_t)stream);
 }
 
 extern "C" int imb_norm_batch_stats(const imb_disc_desc* d, const float* batch, int64_t ld, int64_t n, int row0, int din,
                                     float* norm_state, int32_t* norm_count, float* defer, int defer_cap, float* ws,
                                     void* stream) {
-  cudaStream_t st = (cudaStream_t)stream;
   IMB_REQUIRE(n >= 1 && din >= 1 && din <= IMB_MAX_DIN, "norm batch stats: bad sizes");
   IMB_REQUIRE(defer == nullptr || defer_cap >= 1, "norm batch stats: defer_cap");
-  const WsLayout w = ws_layout(d->n_params);
-  NormLaunch NL;
-  NL.din = din;
-  for (int k = 0; k < din; ++k) NL.row[k] = (short)(row0 + k);
-  const int chunk_rows = n <= (int64_t)128 * 2048 ? 128 : NORM_CHUNK;
-  const int chunks = (int)((n + chunk_rows - 1) / chunk_rows);
-  IMB_REQUIRE(chunks >= 1 && chunks <= MAXCHUNKS, "norm update: n=%lld out of range", (long long)n);
-  k_norm_stats<<<chunks, 256, 0, st>>>(NL, batch, ld, n, chunk_rows, norm_state, norm_count, nullptr, ws + w.normpart,
-                                       reinterpret_cast<unsigned int*>(ws + w.ticket), defer, defer_cap);
-  IMB_CHECK_LAUNCH("k_norm_stats(batch)");
-  return 0;
+  NormJobs J{};
+  J.njobs = 1;
+  J.job[0].din = din;
+  for (int k = 0; k < din; ++k) J.job[0].row[k] = (short)(row0 + k);
+  J.job[0].rmv = norm_state;
+  J.job[0].cnt = norm_count;
+  return norm_stats(J, batch, ld, n, defer, defer_cap, ws, ws_layout(d->n_params), (cudaStream_t)stream);
 }
 
 extern "C" int imb_norm_fold(int din, float* defer, float* norm_state, int32_t* norm_count, int n_slots, void* stream) {
@@ -1325,15 +1197,19 @@ extern "C" int imb_disc_fwd_bwd(const imb_disc_desc* d, const float* params, con
   return 0;
 }
 
+// grid of k_disc_reduce / k_disc_reduce_adam: a warp per parameter and per statistic, at most two 256-thread blocks per SM
+static int reduce_blocks(int P) {
+  const int blocks = ((P + 5) * 32 + 255) / 256;
+  return blocks < 2 * imb_num_sms() ? blocks : 2 * imb_num_sms();
+}
+
 extern "C" int imb_disc_reduce(const imb_disc_desc* d, float* ws, float* grad_out_flat, void* stream) {
   cudaStream_t st = (cudaStream_t)stream;
   const WsLayout w = ws_layout(d->n_params);
   IMB_REQUIRE(g_last_grid > 0, "imb_disc_reduce called before imb_disc_fwd_bwd");
   const int P = d->n_params;
-  const int warps = P + 5;
-  int blocks = (warps * 32 + 255) / 256;
-  if (blocks > 2 * imb_num_sms()) blocks = 2 * imb_num_sms();
-  k_disc_reduce<<<blocks, 256, 0, st>>>(P, g_last_grid, ws + w.partial, ws + w.gacc, ws + w.stats, grad_out_flat);
+  k_disc_reduce<<<reduce_blocks(P), 256, 0, st>>>(P, g_last_grid, ws + w.partial, ws + w.gacc, ws + w.stats,
+                                                   grad_out_flat);
   IMB_CHECK_LAUNCH("k_disc_reduce");
   return 0;
 }
@@ -1359,13 +1235,11 @@ extern "C" int imb_disc_reduce_adam(const imb_disc_desc* d, const imb_adam* opt,
   const WsLayout w = ws_layout(d->n_params);
   IMB_REQUIRE(g_last_grid > 0, "imb_disc_reduce_adam called before imb_disc_fwd_bwd");
   const int P = d->n_params;
-  const int warps = P + 5;
-  int blocks = (warps * 32 + 255) / 256;
-  if (blocks > 2 * imb_num_sms()) blocks = 2 * imb_num_sms();
-  k_disc_reduce_adam<<<blocks, 256, 0, st>>>(P, g_last_grid, ws + w.partial, ws + w.gacc, ws + w.stats, *opt, params,
-                                             exp_avg, exp_avg_sq, grad_div, reinterpret_cast<const int*>(ws + w.meta),
-                                             state + IMB_ST_DISC_STEP, stats_out,
-                                             reinterpret_cast<unsigned int*>(ws + w.ticket) + 8);
+  k_disc_reduce_adam<<<reduce_blocks(P), 256, 0, st>>>(P, g_last_grid, ws + w.partial, ws + w.gacc, ws + w.stats, *opt,
+                                                        params, exp_avg, exp_avg_sq, grad_div,
+                                                        reinterpret_cast<const int*>(ws + w.meta),
+                                                        state + IMB_ST_DISC_STEP, stats_out,
+                                                        reinterpret_cast<unsigned int*>(ws + w.ticket) + 8);
   IMB_CHECK_LAUNCH("k_disc_reduce_adam");
   return 0;
 }

@@ -41,9 +41,9 @@ extern "C" {
 #define IMB_MAX_HIDDEN 64   /* hidden widths 1..64, at most 2 hidden layers */
 #define IMB_MAX_DIN 64      /* MLP input width 1..64 */
 #define IMB_F_ZERO_GRAD 1    /* imb_disc_fwd_bwd: clear the gradient accumulator first */
-#define IMB_F_TRAIN_NORM 2
+#define IMB_F_TRAIN_NORM 2   /* imb_disc_fwd_bwd: Phi(s') uses the mid-update norm snapshot */
 #define IMB_F_NO_TENSOR 4    /* imb_disc_fwd_bwd: force the fp32-FFMA kernel (A/B measurements; default = tcgen05 when the shape fits) */
-#define IMB_RF_DETERMINISTIC 1 /* imb_rollout flags: act = mean / argmax (policy.predict(deterministic=True)) */   /* imb_disc_fwd_bwd: Phi(s') uses the mid-update norm snapshot */
+#define IMB_RF_DETERMINISTIC 1 /* imb_rollout flags: act = mean / argmax (policy.predict(deterministic=True)) */
 
 /* One MLP: [RunningNorm?] -> Linear(din,h1) -> act -> [Linear(h1,h2) -> act] -> Linear(h_last,n_out).
  * util/networks.py:204-283 (build_mlp).  Parameter block (at `param_off` floats into the
